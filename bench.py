@@ -23,7 +23,7 @@ The numerator is the job size as the reference defines it: n_cells * n_days plus
 algorithm requires (365 for the aridity pass + passes * 366 per cell); `config.executed_*` quote the
 cell-days the GPU actually simulated (exact cycle skipping removes work).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--cells C] [--years Y]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--cells C] [--years Y] [--dump-outputs DIR]
 N > 1 is launched by torchrun (one rank per GPU, NCCL); RANK/LOCAL_RANK/WORLD_SIZE come from the env.
 """
 from __future__ import annotations
@@ -51,6 +51,8 @@ GRID_SEED = 20240
 ROW_BLOCK = 8        # grid rows per scheduling block of the strong-scaling shards
 E2E_MAX_STEPS = 3    # timed passes of the host-fed leg (each moves ~220 GB over PCIe at N = 1)
 ROOFLINE_MAX_STEPS = 3
+DUMP_BYTES = 64 * 10**6   # --dump-outputs: at most this much in all
+DUMP_SEED = 20241
 
 
 def fp64_work_per_cell_day():
@@ -77,7 +79,17 @@ def parse_args(argv=None):
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-weak", action="store_true", help="skip the weak-scaling figure at N > 1")
-    return ap.parse_args(argv)
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed (the 9 monthly layers and cell_diag, f64) "
+                         "as DIR/<name>.npy: the columns of a fixed, seeded sample of the cells whose result on the host "
+                         "checker is finite (rank 0's cells at N > 1), and their grid indices as cell_index.npy; "
+                         f"at most {DUMP_BYTES // 10**6} MB in all; not with --impl reference")
+    args = ap.parse_args(argv)
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes what the CUDA path computed: it has no meaning with --impl reference")
+    return args
 
 
 def plan_seconds(args, world: int) -> dict:
@@ -193,6 +205,35 @@ def seg_index(segs) -> np.ndarray:
     return np.concatenate([np.arange(a, b, dtype=np.int64) for a, b in segs]) if segs else np.zeros(0, np.int64)
 
 
+def dump_sample(n_cells: int, values_per_cell: int, finite_of) -> np.ndarray:
+    """Local cell indices written by --dump-outputs, ascending: the first cells, in an order drawn with DUMP_SEED, for
+    which finite_of(ascending local indices) -> bool mask says that their result is finite, as many as fit in DUMP_BYTES
+    (f64, with room for the .npy headers).  finite_of is the host checker (host_finite), so the choice depends on the
+    inputs only and every build writes the same cells.  The reference's own arithmetic overflows to inf in ro / bflow for
+    some very sandy soils (about 0.5 % of the grid: pow(x, 1/lambda) underflows, then exp() overflows); such values
+    cannot be compared within a tolerance."""
+    order = np.random.default_rng(DUMP_SEED).permutation(n_cells)
+    k = min(n_cells, (DUMP_BYTES - 64 * 1024) // (8 * values_per_cell))
+    chosen, pos = [], 0
+    while len(chosen) < k and pos < n_cells:
+        batch = order[pos:pos + (k - len(chosen)) * 51 // 50 + 64]  # ~0.5 % of the cells are dropped
+        pos += len(batch)
+        ok = set(np.sort(batch)[finite_of(np.sort(batch))].tolist())
+        chosen += [c for c in batch.tolist() if c in ok]
+    return np.sort(np.asarray(chosen[:k], dtype=np.int64))
+
+
+def host_finite(grid, index, n_years):
+    """finite_of for dump_sample: which of the local cells `sub` (global cells index[sub]) have a finite result, all
+    monthly layers and cell_diag, on the C restatement of the reference core (tests/oracle_lib.py), on all host cores."""
+    from tests import oracle_lib as ol
+
+    def finite_of(sub):
+        r = ol.run_cpu(host_problem(grid, index[sub], n_years), monthly=True)
+        return np.all([np.isfinite(r[k]).all(0) for k in _abi.OUTPUT_NAMES + ("cell_diag",)], axis=0)
+    return finite_of
+
+
 def grid_in_struct(n_cells, n_days, year, doy, month, sw, tc, pn, cells, mem_kind, f32):
     s = _abi.SplashGridIn()
     s.n_cells, s.n_days, s.cell_stride = n_cells, n_days, n_cells
@@ -227,17 +268,21 @@ def sample_indices(n_cells: int, sample_cells: int) -> np.ndarray:
 
 def cpu_sample_problem(sample_cells, n_years, n_cells=synthetic.N_CELLS_5ARCMIN):
     """The CPU legs' bounded sample: a SUBSET of the benchmark grid (same seed, same generator)."""
-    from tests import oracle_lib as ol
-
     grid = synthetic.Grid(n_cells, GRID_SEED)
     pick = sample_indices(n_cells, sample_cells)
+    return host_problem(grid, pick, n_years), pick
+
+
+def host_problem(grid, pick, n_years):
+    """Host copy (f64) of the inputs of the grid's cells `pick` (global indices, ascending)."""
+    from tests import oracle_lib as ol
+
     cells = grid.cells(pick)
     dates = synthetic.daily_dates(FIRST_YEAR, n_years)
     year, doy, month = _abi.time_axes(dates)
     sw, tc, pn = grid.forcing(cells, doy)
-    prob = ol.GridProblem(year, doy, month, sw, tc, pn, cells["lat"], cells["elev"], cells["slop"], cells["asp"],
+    return ol.GridProblem(year, doy, month, sw, tc, pn, cells["lat"], cells["elev"], cells["slop"], cells["asp"],
                           cells["resolution"], cells["soil"], cells["au"])
-    return prob, pick
 
 
 def time_cpu(prob, core, threads):
@@ -463,6 +508,15 @@ def main():
     launches = int(sum(s["kernel_launches"] for s in stats_steps))
     finite_frac = float(torch.isfinite(outs[0]).double().mean().item())
     phases["value_s"] = time.perf_counter() - t0
+
+    # what the last timed step computed, before the roofline leg below writes into the same buffers
+    if args.dump_outputs and rank == 0:
+        pick = dump_sample(nc, len(outs) * n_out + _abi.SPLASH_NDIAG + 1, host_finite(grid, shard.index, args.years))
+        pt = torch.as_tensor(pick, device=device)
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for k, o in zip(_abi.OUTPUT_NAMES + ("cell_diag",), outs + [diag]):
+            np.save(os.path.join(args.dump_outputs, f"{k}.npy"), o[:, pt].cpu().numpy())
+        np.save(os.path.join(args.dump_outputs, "cell_index.npy"), shard.index[pick].astype(np.float64))  # global grid cells
 
     # GPU results of the parity sample (rank 0, N == 1: the CPU leg runs the same cells on the reference)
     sample_got = None

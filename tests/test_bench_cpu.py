@@ -24,6 +24,37 @@ def test_reference_arm_line():
     assert "workload" in line["config"] and line["gpu_launches"] == 0
 
 
+def test_dump_sample_is_fixed_and_fits_the_cap():
+    """--dump-outputs writes the same cells on every run, only cells the checker calls finite, as many as fit in
+    DUMP_BYTES (f64 + the eleven .npy headers); it asks the checker about each cell at most once."""
+    import numpy as np
+    import pytest
+
+    import bench
+    from rsplash_b200 import _abi, synthetic
+
+    per_cell = 9 * 120 + _abi.SPLASH_NDIAG + 1  # the 10-year workload's monthly layers, cell_diag and the cell index
+    finite = np.ones(synthetic.N_CELLS_5ARCMIN, dtype=bool)
+    finite[::173] = False
+    asked = []
+
+    def finite_of(sub):
+        assert (np.diff(sub) > 0).all()
+        asked.extend(sub.tolist())
+        return finite[sub]
+
+    a = bench.dump_sample(len(finite), per_cell, finite_of)
+    assert len(asked) == len(set(asked)) and len(asked) < 1.05 * len(a) + 200
+    assert np.array_equal(a, bench.dump_sample(len(finite), per_cell, lambda s: finite[s])) and (np.diff(a) > 0).all()
+    assert finite[a].all() and len(a) * per_cell * 8 + 11 * 128 <= bench.DUMP_BYTES
+    assert len(a) == (bench.DUMP_BYTES - 64 * 1024) // (8 * per_cell)
+    assert np.array_equal(bench.dump_sample(1000, per_cell, lambda s: finite[s]), np.flatnonzero(finite[:1000]))
+    with pytest.raises(SystemExit):
+        bench.parse_args(["--steps", "0"])
+    with pytest.raises(SystemExit):
+        bench.parse_args(["--impl", "reference", "--dump-outputs", "x"])
+
+
 def test_cuda_arm_has_no_cpu_fallback():
     import torch
 
