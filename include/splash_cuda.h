@@ -55,7 +55,7 @@
 extern "C" {
 #endif
 
-#define SPLASH_ABI_VERSION 5
+#define SPLASH_ABI_VERSION 6
 #define SPLASH_NSTATE 7
 
 /* status codes */
@@ -296,8 +296,8 @@ int splash_month2day_linear(splash_ctx* ctx, const splash_m2d_in* in, void* dail
  * Small-grid branch of splash.grid (R/splash.grid.R:95-110): resolution <- sqrt(area(elev)) * 1000, lat from the cell
  * centres, terrain(elev, opt = c('slope', 'aspect'), unit = 'degrees') with NA slopes of valid cells set to 0 (:107), and
  * of upslope_area() (R/upslope_area.R:12-58) the flow direction terrain(elev, opt = 'flowdir') and the in-tree focal
- * counts ncellflow(flowdir, 'in' | 'out', met = 'top') (:140-165).  The contributing area itself comes from
- * topmodel::sinkfill / topidx (CRAN, not in the reference tree) and stays with the caller.
+ * counts ncellflow(flowdir, 'in' | 'out', met = 'top') (:140-165).  The contributing area itself (topmodel::sinkfill /
+ * topidx) is splash_upslope_area_run below.
  * PARITY UNPINNED: raster::terrain and raster::area are third-party code that is not in /root/reference; the kernels
  * follow their published formulas (Horn 1981 slope/aspect on 8 neighbours with metric cell sizes from the latitude,
  * D8 flow direction with codes 1 = E, 2 = SE, 4 = S, ... 128 = NE, drop over distance), and where raster is random (ties
@@ -322,6 +322,53 @@ typedef struct splash_terrain_out {  /* every layer [n_rows*n_cols] row-major; a
 } splash_terrain_out;
 
 int splash_terrain_run(splash_ctx* ctx, const splash_terrain_in* in, splash_terrain_out* out);
+
+/* ---- upslope contributing area (SURVEY 8f-2, second slice): the Au layer of splash_grid_in ----
+ * What upslope_area() gets from topmodel::sinkfill(dem, res, degree) and topidx(filled, res)$area
+ * (R/upslope_area.R:12-58): depression filling, then multiple-flow-direction accumulation.  Au[1] of the reference;
+ * Au[2], Au[3] are splash_terrain_run's ncellin / ncellout.
+ *
+ * PARITY UNPINNED: topmodel is CRAN code that is not in the reference tree, so this is a precise published definition:
+ *   Cells.  Per-row metric sizes dx, dy as splash_terrain_run (lonlat: a sphere of 6 378 137 m at the row's centre
+ *     latitude), diagonal distance dd = sqrt(dx^2 + dy^2), cell area dx*dy.  Flow runs between valid cells only, over
+ *     8 neighbours; distances and contour lengths of a step are those of the row the step starts in.
+ *   Boundary.  A valid cell is a boundary cell if it is on the grid edge or has an NA neighbour.
+ *   Fill.  The filled surface W is the least surface with W >= Z, W = Z on boundary cells, and for every other valid
+ *     cell a valid neighbour n with W(c) >= W(n) + eps(c->n), eps = dist(c->n) * tan(min_slope_deg) (Planchon and
+ *     Darboux 2001): the fixpoint of W(c) = max(Z(c), min_n W(n) + eps(c->n)), unique because eps > 0 (and for
+ *     floating point as long as W + eps > W, i.e. eps above half an ulp of the elevations).
+ *   Accumulation.  Quinn et al. (1991), as topidx: every valid neighbour n with W(n) < W(c) receives the share
+ *     w / S of c's area, w = tan(beta) * L, tan(beta) = (W(c) - W(n)) / dist, L = 0.5 r (cardinal) or 0.354 r
+ *     (diagonal), r = sqrt(dx*dy), S the sum of c's w.  area(c) = dx*dy + sum over donors u of area(u) * (w_uc / S_u).
+ *     The area of a cell without a lower valid neighbour leaves the grid there.
+ *   Evaluation order.  Neighbours in D8 code order (E, SE, S, SW, W, NW, N, NE) for both sums, each a left-to-right
+ *     sum starting from 0 (S) or dx*dy (area); w = ((W(c) - W(n)) / dist) * L.  tan(), cos() and every per-row value
+ *     are computed once on the host; the kernels use no FMA and IEEE division, so the result is reproducible bit
+ *     for bit and does not depend on the schedule.
+ * To be checked against a real R run of upslope_area(): the 0.354 literal for the diagonal contour length; per-row
+ * metric cell sizes (topmodel takes one square `res`); the edge and NA treatment (R/upslope_area.R sets NA to -9999
+ * before the call); and the `degree` R passes to sinkfill (0.1 is assumed, also the Python default).
+ *
+ * Elevations must be finite or NaN (+-inf is SPLASH_ERR_BAD_ARG); n_rows * n_cols must fit in int32 and n_rows in
+ * 2 097 120.  The fill runs at most n_rows * n_cols sweeps and the accumulation at most one round per valid cell;
+ * reaching either bound is SPLASH_ERR_CUDA, not a loop.  Multi-GPU contexts run it on their first GPU. */
+typedef struct splash_upslope_in {
+    int64_t n_rows, n_cols;
+    const double* elev;     /* [n_rows*n_cols] row-major, north row first; NaN = NA (as splash_terrain_in) */
+    double ymax, xres, yres;/* as splash_terrain_in */
+    int32_t lonlat;
+    int32_t mem_kind;       /* SPLASH_MEM_HOST or SPLASH_MEM_DEVICE, inputs and outputs alike */
+    double min_slope_deg;   /* minimum drop the fill enforces, degrees, in (0, 90) (topmodel::sinkfill's `degree`) */
+} splash_upslope_in;
+
+typedef struct splash_upslope_out {
+    double* area;           /* [n_rows*n_cols] contributing area m2 (own cell included); NA where elev is NA */
+    double* filled;         /* optional [n_rows*n_cols]: the filled DEM W (NULL = not wanted) */
+    int64_t fill_sweeps;    /* written by the call: global fill sweeps run, the last of which changed no cell */
+    int64_t accum_rounds;   /* written by the call: accumulation rounds (= cells on the longest flow path) */
+} splash_upslope_out;
+
+int splash_upslope_area_run(splash_ctx* ctx, const splash_upslope_in* in, splash_upslope_out* out);
 
 /* Diagnostic (used by tests/test_math_gpu.py, not by the R glue): apply one of the day step's
  * transcendental functions to a host array on the device.  op: 0 exp, 1 log, 2 acos, 3 sin (hour

@@ -5,8 +5,8 @@
 return the same nine layers (R/splash.grid.R:449).  They only marshal numpy arrays into the C ABI
 (include/splash_cuda.h); all arithmetic happens in libsplash_cuda's CUDA kernels.
 
-What stays outside (as in the survey's scope table): raster I/O, terrain derivation (slope,
-aspect, upslope area, latitude, resolution are *inputs* here, as they are for splash.point), and
+What stays outside (as in the survey's scope table): raster I/O (slope, aspect, upslope area, latitude and
+resolution are *inputs* of splash_grid, as they are for splash.point; `terrain` and `upslope_area` derive them), and
 the random monthly->daily rain disaggregation (the deterministic interpolation of monthly temperature and
 radiation is `month2day_linear`).
 """
@@ -207,6 +207,68 @@ def terrain(elev, ymax: float, xres: float, yres: float, lonlat: bool = True, ct
     for k, v in res.items():
         setattr(cout, k, _ptr(v))
     ctx.check(ctx.lib.splash_terrain_run(ctx.handle, C.byref(cin), C.byref(cout)))
+    return res
+
+
+def upslope_area(elev, ymax: float, xres: float, yres: float, lonlat: bool = True, min_slope_deg: float = 0.1,
+                 ctx: Context | None = None, return_filled: bool = False, in_ptr: int | None = None,
+                 out_ptr: int | None = None, filled_ptr: int | None = None, shape: tuple | None = None) -> dict:
+    """upslope_area() of the reference (R/upslope_area.R:12-58, small-grid branch): the contributing area of every cell
+    (topmodel::sinkfill, then topidx's multiple-flow-direction area; see include/splash_cuda.h for the definition,
+    PARITY UNPINNED) and the in / out neighbour counts of splash_terrain_run.
+
+    elev  [n_rows, n_cols], north row first, NaN = NA;  min_slope_deg  the fill's minimum slope (sinkfill's `degree`).
+    Returns {area, ncellin, ncellout, Au, fill_sweeps, accum_rounds[, filled]}: Au is the [3, n_rows, n_cols] stack
+    (area m2, ncellin, ncellout) that splash_grid takes per cell, and area / ncellin / ncellout are its layers.
+    With in_ptr / out_ptr (device addresses of the [n_rows, n_cols] float64 DEM and of a [3, n_rows, n_cols] float64
+    array that receives Au, e.g. torch tensors' data_ptr()) and shape = (n_rows, n_cols), everything stays in HBM
+    (filled_ptr: optional [n_rows, n_cols] float64 for the filled DEM) and only the two counters are returned.
+    """
+    ctx = ctx or default_context()
+    if (in_ptr is None) != (out_ptr is None):
+        raise ValueError("in_ptr and out_ptr go together")
+    device = in_ptr is not None
+    if device:
+        if shape is None:
+            raise ValueError("shape is required with device pointers")
+        nr, nc = (int(s) for s in shape)
+    else:
+        z = np.ascontiguousarray(elev, dtype=np.float64)
+        if z.ndim != 2:
+            raise ValueError("elev must be [n_rows, n_cols]")
+        nr, nc = z.shape
+        au = np.empty((3, nr, nc))
+        filled = np.empty((nr, nc)) if return_filled else None
+    n = nr * nc
+    mem = _abi.SPLASH_MEM_DEVICE if device else _abi.SPLASH_MEM_HOST
+    elev_p = C.c_void_p(int(in_ptr)) if device else _ptr(z)
+    au_addr = int(out_ptr) if device else au.ctypes.data
+    layer = lambda k: C.c_void_p(au_addr + k * n * 8) if n else None
+
+    cin = _abi.SplashUpslopeIn()
+    cin.n_rows, cin.n_cols, cin.elev = nr, nc, elev_p
+    cin.ymax, cin.xres, cin.yres, cin.lonlat, cin.mem_kind = float(ymax), float(xres), float(yres), int(bool(lonlat)), mem
+    cin.min_slope_deg = float(min_slope_deg)
+    cout = _abi.SplashUpslopeOut()
+    cout.area = layer(0)
+    if device:
+        cout.filled = None if filled_ptr is None else C.c_void_p(int(filled_ptr))
+    else:
+        cout.filled = _ptr(filled)
+    ctx.check(ctx.lib.splash_upslope_area_run(ctx.handle, C.byref(cin), C.byref(cout)))
+
+    tin = _abi.SplashTerrainIn()
+    tin.n_rows, tin.n_cols, tin.elev = nr, nc, elev_p
+    tin.ymax, tin.xres, tin.yres, tin.lonlat, tin.mem_kind = cin.ymax, cin.xres, cin.yres, cin.lonlat, mem
+    tout = _abi.SplashTerrainOut()
+    tout.ncellin, tout.ncellout = layer(1), layer(2)
+    ctx.check(ctx.lib.splash_terrain_run(ctx.handle, C.byref(tin), C.byref(tout)))
+
+    res = {"fill_sweeps": int(cout.fill_sweeps), "accum_rounds": int(cout.accum_rounds)}
+    if not device:
+        res.update(area=au[0], ncellin=au[1], ncellout=au[2], Au=au)
+        if return_filled:
+            res["filled"] = filled
     return res
 
 

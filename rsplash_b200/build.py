@@ -10,7 +10,7 @@ CSRC = os.path.join(PKG_DIR, "csrc")
 # SPLASH_CUDA_LIB: development override to load/build a variant of the library (e.g. another SPLASH_LEVEL)
 LIB_PATH = os.environ.get("SPLASH_CUDA_LIB") or os.path.join(PKG_DIR, "libsplash_cuda.so")
 SOURCES = [os.path.join(CSRC, "splash_cuda.cu")]
-HEADERS = [os.path.join(CSRC, "splash_model.cuh"), os.path.join(CSRC, "splash_math.cuh"), os.path.join(CSRC, "splash_consts.cuh"), os.path.join(CSRC, "splash_host_tables.h"), os.path.join(PKG_DIR, "..", "include", "splash_cuda.h")]
+HEADERS = [os.path.join(CSRC, "splash_model.cuh"), os.path.join(CSRC, "splash_math.cuh"), os.path.join(CSRC, "splash_consts.cuh"), os.path.join(CSRC, "splash_host_tables.h"), os.path.join(CSRC, "splash_upslope.cuh"),os.path.join(PKG_DIR, "..", "include", "splash_cuda.h")]
 
 # -fmad=false: the reference build has no FMA contraction (R's default x86-64 flags); the day step
 # mirrors its evaluation order, explicit fma() is used only where glibc's expf does.

@@ -47,6 +47,7 @@
 
 #include "splash_model.cuh"
 #include "splash_host_tables.h"
+#include "splash_upslope.cuh"
 
 using namespace splash;
 
@@ -2185,6 +2186,162 @@ int splash_terrain_run(splash_ctx* ctx, const splash_terrain_in* in, splash_terr
     if (in->mem_kind == SPLASH_MEM_HOST)
         for (int k = 0; k < 7; ++k)
             if (optr[k]) CU(cudaMemcpyAsync(optr[k], *slot[k], (size_t)n * 8, cudaMemcpyDeviceToHost, S));
+    CU(cudaStreamSynchronize(S));
+    return SPLASH_OK;
+}
+
+// Per-row metrics of the upslope area (splash_upslope.cuh: UR_*), on the host with libm so that the kernels and a
+// numpy restatement (Python's math module is the same libm) share every operand.  No contraction into FMA.
+__attribute__((optimize("fp-contract=off"))) static void upslope_rows(const splash_upslope_in* in, std::vector<double>& rows) {
+    using namespace upslope;
+    const double t = tan(in->min_slope_deg * kpir);
+    rows.resize((size_t)in->n_rows * UR_N);
+    for (int64_t r = 0; r < in->n_rows; ++r) {
+        double* m = rows.data() + r * UR_N;
+        const double lat_c = in->ymax - ((double)r + 0.5) * in->yres;
+        const double dy = in->lonlat ? kEarthR * (in->yres * kpir) : in->yres;
+        const double dx = in->lonlat ? kEarthR * cos(lat_c * kpir) * (in->xres * kpir) : in->xres;
+        const double dd = sqrt(dx * dx + dy * dy);
+        const double rl = sqrt(dx * dy);
+        m[UR_DX] = dx;
+        m[UR_DY] = dy;
+        m[UR_DD] = dd;
+        m[UR_AREA] = dx * dy;
+        m[UR_LC] = 0.5 * rl;
+        m[UR_LD] = 0.354 * rl;
+        m[UR_EX] = dx * t;
+        m[UR_EY] = dy * t;
+        m[UR_ED] = dd * t;
+    }
+}
+
+int splash_upslope_area_run(splash_ctx* ctx, const splash_upslope_in* in, splash_upslope_out* out) {
+    using namespace upslope;
+    if (ctx && ctx->multi) {  // single-GPU work: the context's first lane does it
+        splash_ctx* lane = first_lane(ctx);
+        const int rc = splash_upslope_area_run(lane, in, out);
+        ctx->err = lane->err;
+        return rc;
+    }
+    if (!ctx) return SPLASH_ERR_BAD_ARG;
+    ctx->err.clear();
+    if (!in || !out) return fail(ctx, SPLASH_ERR_BAD_ARG, "splash_upslope_area_run: NULL in/out");
+    out->fill_sweeps = 0;
+    out->accum_rounds = 0;
+    const int64_t nr = in->n_rows, ncol = in->n_cols;
+    if (nr < 0 || ncol < 0 || nr > (int64_t)kFT * 65535 || (ncol > 0 && nr > INT32_MAX / ncol))
+        return fail(ctx, SPLASH_ERR_BAD_ARG, "bad n_rows/n_cols (n_rows*n_cols must fit in int32, n_rows <= %d)", kFT * 65535);
+    if (in->mem_kind != SPLASH_MEM_HOST && in->mem_kind != SPLASH_MEM_DEVICE)
+        return fail(ctx, SPLASH_ERR_BAD_ARG, "mem_kind must be SPLASH_MEM_HOST or SPLASH_MEM_DEVICE");
+    if (!(in->xres > 0) || !(in->yres > 0) || !std::isfinite(in->xres) || !std::isfinite(in->yres))
+        return fail(ctx, SPLASH_ERR_BAD_ARG, "xres and yres must be positive and finite");
+    if (!std::isfinite(in->min_slope_deg) || !(in->min_slope_deg > 0.0) || !(in->min_slope_deg < 90.0))
+        return fail(ctx, SPLASH_ERR_BAD_ARG, "min_slope_deg must be in (0, 90)");
+    if (in->lonlat && !(in->ymax <= 90.0 && in->ymax - (double)nr * in->yres >= -90.0))
+        return fail(ctx, SPLASH_ERR_BAD_ARG, "lonlat: the rows must lie between -90 and 90 degrees");
+    const int64_t n = nr * ncol;
+    if (n == 0) return SPLASH_OK;
+    if (!in->elev || !out->area) return fail(ctx, SPLASH_ERR_BAD_ARG, "NULL elev/area");
+    CU(cudaSetDevice(ctx->device));
+    cudaStream_t S = ctx->s_run[0];
+    std::vector<double> rows;
+    upslope_rows(in, rows);
+    const size_t nb = (size_t)n * 8;
+    TmpDev t_z, t_w0, t_w1, t_s, t_area, t_ndon, t_f0, t_f1, t_rows, t_ctl;  // freed on every return path
+    const bool host = in->mem_kind == SPLASH_MEM_HOST;
+    if (host) {
+        CU(cudaMalloc(&t_z.p, nb));
+        CU(cudaMalloc(&t_area.p, nb));
+        CU(cudaMemcpyAsync(t_z.p, in->elev, nb, cudaMemcpyHostToDevice, S));
+    }
+    CU(cudaMalloc(&t_w0.p, nb));
+    CU(cudaMalloc(&t_w1.p, nb));
+    CU(cudaMalloc(&t_s.p, nb));
+    CU(cudaMalloc(&t_ndon.p, (size_t)n * 4));
+    CU(cudaMalloc(&t_f0.p, (size_t)n * 4));
+    CU(cudaMalloc(&t_f1.p, (size_t)n * 4));
+    CU(cudaMalloc(&t_rows.p, rows.size() * 8));
+    constexpr int kMaxBatch = 64;  // fill sweeps launched between two reads of their flags
+    CU(cudaMalloc(&t_ctl.p, (AC_N + 1 + kMaxBatch) * sizeof(int)));
+    CU(cudaMemcpyAsync(t_rows.p, rows.data(), rows.size() * 8, cudaMemcpyHostToDevice, S));
+    int* ctl = (int*)t_ctl.p;
+    int* flags = ctl + AC_N;  // flags[0]: "the sweep before this batch changed something"; flags[1..batch]: the batch
+    CU(cudaMemsetAsync(ctl, 0, AC_N * sizeof(int), S));
+    const double* z = host ? (const double*)t_z.p : in->elev;
+    double* area = host ? (double*)t_area.p : out->area;
+    double* w[2] = {(double*)t_w0.p, (double*)t_w1.p};
+    FillParams fp{z, (const double*)t_rows.p, (int)nr, (int)ncol};
+    const unsigned grid = (unsigned)((n + 255) / 256);
+    k_fill_init<<<grid, 256, 0, S>>>(fp, w[0], ctl + AC_BADZ, ctl + AC_NVALID);
+    CU(cudaGetLastError());
+    int hctl[AC_N + 1 + kMaxBatch];
+    CU(cudaMemcpyAsync(hctl, ctl, AC_N * sizeof(int), cudaMemcpyDeviceToHost, S));
+    CU(cudaStreamSynchronize(S));
+    if (hctl[AC_BADZ]) return fail(ctx, SPLASH_ERR_BAD_ARG, "splash_upslope_area_run: elev has +-inf values (NaN is NA)");
+
+    // fill: batches of sweeps between reads of the flags (no host round trip per sweep); bound n sweeps
+    const dim3 fgrid((unsigned)((ncol + kFT - 1) / kFT), (unsigned)((nr + kFT - 1) / kFT)), fblock(kFT, kFRows);
+    int64_t sweeps = 0;
+    bool converged = false;
+    for (int batch = 4; !converged;) {
+        const int one = 1;
+        CU(cudaMemcpyAsync(flags, &one, sizeof(int), cudaMemcpyHostToDevice, S));
+        CU(cudaMemsetAsync(flags + 1, 0, batch * sizeof(int), S));
+        for (int j = 1; j <= batch; ++j) {
+            const int64_t s = sweeps + j - 1;
+            k_fill_sweep<<<fgrid, fblock, 0, S>>>(fp, w[s & 1], w[(s + 1) & 1], flags, j);
+        }
+        CU(cudaGetLastError());
+        CU(cudaMemcpyAsync(hctl, flags + 1, batch * sizeof(int), cudaMemcpyDeviceToHost, S));
+        CU(cudaStreamSynchronize(S));
+        for (int j = 0; j < batch && !converged; ++j) {
+            ++sweeps;
+            converged = hctl[j] == 0;
+        }
+        if (!converged && sweeps >= n)
+            return fail(ctx, SPLASH_ERR_CUDA, "splash_upslope_area_run: the fill did not converge in %lld sweeps", (long long)n);
+        batch = std::min(2 * batch, kMaxBatch);
+    }
+    out->fill_sweeps = sweeps;
+    const double* wf = w[sweeps & 1];  // written by the last sweep (equal to its input: nothing changed)
+
+    // accumulation
+    AccumParams ap{};
+    ap.w = wf;
+    ap.rows = (const double*)t_rows.p;
+    ap.s = (double*)t_s.p;
+    ap.area = area;
+    ap.ndon = (int*)t_ndon.p;
+    ap.front[0] = (int*)t_f0.p;
+    ap.front[1] = (int*)t_f1.p;
+    ap.ctl = ctl;
+    ap.n_rows = (int)nr;
+    ap.n_cols = (int)ncol;
+    k_flow_prep<<<grid, 256, 0, S>>>(ap);
+    CU(cudaGetLastError());
+    int per_sm = 0;
+    CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_accum, kAccThreads, 0));
+    if (per_sm < 1) return fail(ctx, SPLASH_ERR_CUDA, "splash_upslope_area_run: k_accum does not fit an SM");
+    const unsigned agrid = (unsigned)std::max<int64_t>(1, std::min<int64_t>((int64_t)per_sm * ctx->sm_count, (n + kAccThreads - 1) / kAccThreads));
+    void* args[] = {&ap};
+    // a launch that does not finish runs at least one round, and there are at most n rounds
+    int64_t launches = 0;
+    for (int batch = 2;; batch = std::min(2 * batch, 16)) {
+        if (launches > n + 1) return fail(ctx, SPLASH_ERR_CUDA, "splash_upslope_area_run: the accumulation did not finish");
+        for (int j = 0; j < batch; ++j) CU(cudaLaunchCooperativeKernel((const void*)k_accum, agrid, kAccThreads, args, 0, S));
+        launches += batch;
+        CU(cudaMemcpyAsync(hctl, ctl, AC_N * sizeof(int), cudaMemcpyDeviceToHost, S));
+        CU(cudaStreamSynchronize(S));
+        if (hctl[AC_ERR]) return fail(ctx, SPLASH_ERR_CUDA, "splash_upslope_area_run: more accumulation rounds than valid cells");
+        if (hctl[AC_DONE]) break;
+    }
+    out->accum_rounds = hctl[AC_ROUNDS];
+    if (host) {
+        CU(cudaMemcpyAsync(out->area, area, nb, cudaMemcpyDeviceToHost, S));
+        if (out->filled) CU(cudaMemcpyAsync(out->filled, wf, nb, cudaMemcpyDeviceToHost, S));
+    } else if (out->filled) {
+        CU(cudaMemcpyAsync(out->filled, wf, nb, cudaMemcpyDeviceToDevice, S));
+    }
     CU(cudaStreamSynchronize(S));
     return SPLASH_OK;
 }
