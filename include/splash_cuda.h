@@ -55,7 +55,7 @@
 extern "C" {
 #endif
 
-#define SPLASH_ABI_VERSION 6
+#define SPLASH_ABI_VERSION 7
 #define SPLASH_NSTATE 7
 
 /* status codes */
@@ -369,6 +369,77 @@ typedef struct splash_upslope_out {
 } splash_upslope_out;
 
 int splash_upslope_area_run(splash_ctx* ctx, const splash_upslope_in* in, splash_upslope_out* out);
+
+/* ---- D-infinity contributing area (SURVEY 8f-2, third slice): Au for coarse or large grids ----
+ * What upslope_areav2() (R/upslope_area.R:59-137) gets from TauDEM through mpiexec (:76-81): PitRemove, DinfFlowDir
+ * (which resolves flats) and AreaDinf.  Same cells, boundary and output as splash_upslope_area_run; the Python
+ * api.upslope_areav2 adds splash_terrain_run's ncellin / ncellout as Au[2], Au[3].
+ *
+ * PARITY UNPINNED: TauDEM and the lines of R/upslope_area.R that call it are not in this tree, so this is a precise
+ * published definition:
+ *   Cells, distances, boundary.  As splash_upslope_area_run: per-row dx, dy, dd = sqrt(dx^2 + dy^2), area dx*dy, the
+ *     metrics of a step taken from the row it starts in; a boundary cell is a valid cell on the grid edge or next to
+ *     an NA cell.
+ *   Fill.  W(c) = the least, over 8-connected paths of valid cells from c to a boundary cell, of the highest Z on the
+ *     path (the minimax spill elevation; W = Z on boundary cells).  It is the greatest solution of
+ *     W(c) = max(Z(c), min_n W(n)), the Planchon-Darboux fixpoint with eps = 0, which the sweeps reach from above.
+ *   Directions.  Boundary cells have none: their area leaves the grid (as TauDEM leaves edge cells without one).  Every
+ *     other valid cell with a strictly lower neighbour takes the D-infinity facet rule on W (Tarboton 1997).  Facets in
+ *     Tarboton's order, (cardinal e1, diagonal e2, ac, af): 1 (E, NE, 0, 1), 2 (N, NE, 1, -1), 3 (N, NW, 1, 1),
+ *     4 (W, NW, 2, -1), 5 (W, SW, 2, 1), 6 (S, SW, 3, -1), 7 (S, SE, 3, 1), 8 (E, SE, 4, -1).  d1, d2 = dx, dy when
+ *     e1 is E or W, dy, dx when it is N or S; theta_f = atan2(d2, d1), per row on the host.
+ *     s1 = (e0 - e1) / d1, s2 = (e1 - e2) / d2, then, by comparisons only:
+ *       s2 > 0, s1 > 0 and s2 * d1 < s1 * d2:  inside the facet, s = sqrt(s1*s1 + s2*s2), r = atan(s2 / s1);
+ *       otherwise s2 > 0:                       clipped to the diagonal, s = (e0 - e2) / dd, r = theta_f;
+ *       otherwise:                              clipped to the cardinal, s = s1, r = 0.
+ *     The facet of largest s > 0 wins, ties to the lowest facet.  Angle = ac * (pi/2) + af * r (2 pi is reported as
+ *     0).  atan(s2 / s1) is the only transcendental the device evaluates.
+ *   Proportions.  Inside a facet the cardinal receiver gets 1 - p and the diagonal one p = min(r / theta_f, 1)
+ *     (TauDEM's angle split for square cells, its natural generalisation for others; the min keeps a share from going
+ *     negative when atan rounds r a few ulp past theta_f); a clipped cell has one receiver, with 1.
+ *   Flats.  A flat cell is a valid non-boundary cell without a strictly lower neighbour.  Each 8-connected set of flat
+ *     cells is level and has an outlet: a non-flat or boundary neighbour at the same W.  Flats are resolved as
+ *     Garbrecht and Martz (1997) in the formulation of Barnes, Lehman and Mulla (2014): breadth-first distances
+ *     towards lower (1 next to an outlet) and away from higher (1 on flat cells next to higher ground), H = the
+ *     largest away distance of the flat (0, with away = 0, on a flat without higher ground), and the mask
+ *     M = 2 * towards + (H - away); outlets count as M = 0.  A flat cell takes the facet rule on M instead of W, over
+ *     the facets whose two neighbours are at its W.  If no facet gives s > 0, everything goes to the neighbour at its W
+ *     of steepest descent (M(c) - M(n)) / dist, ties to the lowest D8 code, with the angle of the first facet that has
+ *     that neighbour, clipped to it (Barnes: such a neighbour exists).
+ *   Accumulation.  area(c) = dx*dy + sum over donors u in D8 code order of area(u) * p(u->c), a left-to-right sum,
+ *     no FMA, IEEE division.  Every receiver is strictly lower in W or, on a flat, in M, so the graph is acyclic and
+ *     the result does not depend on the schedule.
+ * To be checked against a real R + TauDEM run of upslope_areav2(), in this order:
+ *   1. which TauDEM tool's grid becomes Au[1] (AreaDinf's is assumed, not AreaD8's);
+ *   2. the conversion of TauDEM's specific catchment area (per unit contour width) to m2 (here: the area itself);
+ *   3. edge contamination: assumed off, i.e. the area is reported everywhere, as TauDEM's -nc;
+ *   4. that edge cells have no direction;
+ *   5. the proportion rule on non-square cells;
+ *   6. the weighting of the two gradients of Garbrecht and Martz: TauDEM's own flat code may weight them otherwise;
+ *   7. that Au[2..3] are still ncellflow's counts.
+ *
+ * Arguments, limits and multi-GPU contexts as splash_upslope_area_run.  The fill and the flat labelling run at most
+ * n_rows * n_cols sweeps each, the distances and the accumulation at most one round per valid cell; reaching a bound
+ * is SPLASH_ERR_CUDA, not a loop. */
+typedef struct splash_dinf_in {
+    int64_t n_rows, n_cols;
+    const double* elev;     /* as splash_upslope_in */
+    double ymax, xres, yres;
+    int32_t lonlat;
+    int32_t mem_kind;       /* SPLASH_MEM_HOST or SPLASH_MEM_DEVICE, inputs and outputs alike */
+} splash_dinf_in;
+
+typedef struct splash_dinf_out {
+    double* area;           /* [n_rows*n_cols] contributing area m2 (own cell included); NA where elev is NA */
+    double* filled;         /* optional [n_rows*n_cols]: the filled DEM W (NULL = not wanted) */
+    double* angle;          /* optional [n_rows*n_cols]: flow angle, radians counter-clockwise from east in [0, 2 pi);
+                               NaN where a cell has no direction */
+    int64_t fill_sweeps;    /* written by the call: global fill sweeps run, the last of which changed no cell */
+    int64_t flat_rounds;    /* written by the call: flat labelling sweeps + rounds of the two distances */
+    int64_t accum_rounds;   /* written by the call: accumulation rounds (= cells on the longest flow path) */
+} splash_dinf_out;
+
+int splash_upslope_dinf_run(splash_ctx* ctx, const splash_dinf_in* in, splash_dinf_out* out);
 
 /* Diagnostic (used by tests/test_math_gpu.py, not by the R glue): apply one of the day step's
  * transcendental functions to a host array on the device.  op: 0 exp, 1 log, 2 acos, 3 sin (hour

@@ -9,7 +9,7 @@ import ctypes as C
 
 import numpy as np
 
-SPLASH_ABI_VERSION = 6
+SPLASH_ABI_VERSION = 7
 SPLASH_NSTATE = 7
 
 SPLASH_OK, SPLASH_ERR_BAD_ARG, SPLASH_ERR_CUDA, SPLASH_ERR_NOMEM, SPLASH_ERR_NO_DEVICE = range(5)
@@ -134,6 +134,18 @@ class SplashUpslopeIn(C.Structure):
 
 class SplashUpslopeOut(C.Structure):
     _fields_ = [("area", C.c_void_p), ("filled", C.c_void_p), ("fill_sweeps", C.c_int64), ("accum_rounds", C.c_int64)]
+
+
+class SplashDinfIn(C.Structure):
+    _fields_ = [
+        ("n_rows", C.c_int64), ("n_cols", C.c_int64), ("elev", C.c_void_p), ("ymax", C.c_double), ("xres", C.c_double),
+        ("yres", C.c_double), ("lonlat", C.c_int32), ("mem_kind", C.c_int32),
+    ]
+
+
+class SplashDinfOut(C.Structure):
+    _fields_ = [("area", C.c_void_p), ("filled", C.c_void_p), ("angle", C.c_void_p), ("fill_sweeps", C.c_int64),
+                ("flat_rounds", C.c_int64), ("accum_rounds", C.c_int64)]
 
 
 class SplashStats(C.Structure):

@@ -15,7 +15,7 @@ EXPORTS = (
     "splash_abi_version", "splash_ctx_create", "splash_ctx_destroy", "splash_last_error", "splash_count_months",
     "splash_grid_run", "splash_point_run", "splash_last_stats", "splash_debug_math", "splash_unswc_grid_run",
     "splash_month2day_linear", "splash_ctx_create_multi", "splash_ctx_device_count", "splash_cluster_create",
-    "splash_terrain_run", "splash_upslope_area_run", "splash_cluster_destroy", "splash_cluster_lanes", "splash_cluster_submit", "splash_cluster_wait", "splash_cluster_last_error",
+    "splash_terrain_run", "splash_upslope_area_run", "splash_upslope_dinf_run", "splash_cluster_destroy", "splash_cluster_lanes", "splash_cluster_submit", "splash_cluster_wait", "splash_cluster_last_error",
 )
 
 _lib = None
@@ -66,6 +66,8 @@ def load() -> C.CDLL:
     lib.splash_terrain_run.restype = C.c_int
     lib.splash_upslope_area_run.argtypes = [C.c_void_p, C.POINTER(_abi.SplashUpslopeIn), C.POINTER(_abi.SplashUpslopeOut)]
     lib.splash_upslope_area_run.restype = C.c_int
+    lib.splash_upslope_dinf_run.argtypes = [C.c_void_p, C.POINTER(_abi.SplashDinfIn), C.POINTER(_abi.SplashDinfOut)]
+    lib.splash_upslope_dinf_run.restype = C.c_int
     lib.splash_ctx_create_multi.argtypes = [C.POINTER(C.c_int), C.c_int, C.POINTER(C.c_void_p)]
     lib.splash_ctx_create_multi.restype = C.c_int
     lib.splash_ctx_device_count.argtypes = [C.c_void_p]

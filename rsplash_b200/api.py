@@ -210,20 +210,10 @@ def terrain(elev, ymax: float, xres: float, yres: float, lonlat: bool = True, ct
     return res
 
 
-def upslope_area(elev, ymax: float, xres: float, yres: float, lonlat: bool = True, min_slope_deg: float = 0.1,
-                 ctx: Context | None = None, return_filled: bool = False, in_ptr: int | None = None,
-                 out_ptr: int | None = None, filled_ptr: int | None = None, shape: tuple | None = None) -> dict:
-    """upslope_area() of the reference (R/upslope_area.R:12-58, small-grid branch): the contributing area of every cell
-    (topmodel::sinkfill, then topidx's multiple-flow-direction area; see include/splash_cuda.h for the definition,
-    PARITY UNPINNED) and the in / out neighbour counts of splash_terrain_run.
-
-    elev  [n_rows, n_cols], north row first, NaN = NA;  min_slope_deg  the fill's minimum slope (sinkfill's `degree`).
-    Returns {area, ncellin, ncellout, Au, fill_sweeps, accum_rounds[, filled]}: Au is the [3, n_rows, n_cols] stack
-    (area m2, ncellin, ncellout) that splash_grid takes per cell, and area / ncellin / ncellout are its layers.
-    With in_ptr / out_ptr (device addresses of the [n_rows, n_cols] float64 DEM and of a [3, n_rows, n_cols] float64
-    array that receives Au, e.g. torch tensors' data_ptr()) and shape = (n_rows, n_cols), everything stays in HBM
-    (filled_ptr: optional [n_rows, n_cols] float64 for the filled DEM) and only the two counters are returned.
-    """
+def _upslope_au(entry, cin, cout, counters, optional, elev, ymax, xres, yres, lonlat, ctx, in_ptr, out_ptr, shape) -> dict:
+    """The marshalling upslope_area and upslope_areav2 share: fill the geometry of `cin` and cout.area, pass the
+    optional [n_rows, n_cols] outputs {field: (wanted on the host, device address or None)}, call `entry`, then
+    splash_terrain_run for the two count layers of Au."""
     ctx = ctx or default_context()
     if (in_ptr is None) != (out_ptr is None):
         raise ValueError("in_ptr and out_ptr go together")
@@ -238,24 +228,22 @@ def upslope_area(elev, ymax: float, xres: float, yres: float, lonlat: bool = Tru
             raise ValueError("elev must be [n_rows, n_cols]")
         nr, nc = z.shape
         au = np.empty((3, nr, nc))
-        filled = np.empty((nr, nc)) if return_filled else None
+        extra = {k: np.empty((nr, nc)) for k, (want, _) in optional.items() if want}
     n = nr * nc
     mem = _abi.SPLASH_MEM_DEVICE if device else _abi.SPLASH_MEM_HOST
     elev_p = C.c_void_p(int(in_ptr)) if device else _ptr(z)
     au_addr = int(out_ptr) if device else au.ctypes.data
     layer = lambda k: C.c_void_p(au_addr + k * n * 8) if n else None
 
-    cin = _abi.SplashUpslopeIn()
     cin.n_rows, cin.n_cols, cin.elev = nr, nc, elev_p
     cin.ymax, cin.xres, cin.yres, cin.lonlat, cin.mem_kind = float(ymax), float(xres), float(yres), int(bool(lonlat)), mem
-    cin.min_slope_deg = float(min_slope_deg)
-    cout = _abi.SplashUpslopeOut()
     cout.area = layer(0)
-    if device:
-        cout.filled = None if filled_ptr is None else C.c_void_p(int(filled_ptr))
-    else:
-        cout.filled = _ptr(filled)
-    ctx.check(ctx.lib.splash_upslope_area_run(ctx.handle, C.byref(cin), C.byref(cout)))
+    for k, (_, dptr) in optional.items():
+        if device:
+            setattr(cout, k, None if dptr is None else C.c_void_p(int(dptr)))
+        else:
+            setattr(cout, k, _ptr(extra.get(k)))
+    ctx.check(getattr(ctx.lib, entry)(ctx.handle, C.byref(cin), C.byref(cout)))
 
     tin = _abi.SplashTerrainIn()
     tin.n_rows, tin.n_cols, tin.elev = nr, nc, elev_p
@@ -264,12 +252,49 @@ def upslope_area(elev, ymax: float, xres: float, yres: float, lonlat: bool = Tru
     tout.ncellin, tout.ncellout = layer(1), layer(2)
     ctx.check(ctx.lib.splash_terrain_run(ctx.handle, C.byref(tin), C.byref(tout)))
 
-    res = {"fill_sweeps": int(cout.fill_sweeps), "accum_rounds": int(cout.accum_rounds)}
+    res = {k: int(getattr(cout, k)) for k in counters}
     if not device:
-        res.update(area=au[0], ncellin=au[1], ncellout=au[2], Au=au)
-        if return_filled:
-            res["filled"] = filled
+        res.update(area=au[0], ncellin=au[1], ncellout=au[2], Au=au, **extra)
     return res
+
+
+def upslope_area(elev, ymax: float, xres: float, yres: float, lonlat: bool = True, min_slope_deg: float = 0.1,
+                 ctx: Context | None = None, return_filled: bool = False, in_ptr: int | None = None,
+                 out_ptr: int | None = None, filled_ptr: int | None = None, shape: tuple | None = None) -> dict:
+    """upslope_area() of the reference (R/upslope_area.R:12-58, small-grid branch): the contributing area of every cell
+    (topmodel::sinkfill, then topidx's multiple-flow-direction area; see include/splash_cuda.h for the definition,
+    PARITY UNPINNED) and the in / out neighbour counts of splash_terrain_run.
+
+    elev  [n_rows, n_cols], north row first, NaN = NA;  min_slope_deg  the fill's minimum slope (sinkfill's `degree`).
+    Returns {area, ncellin, ncellout, Au, fill_sweeps, accum_rounds[, filled]}: Au is the [3, n_rows, n_cols] stack
+    (area m2, ncellin, ncellout) that splash_grid takes per cell, and area / ncellin / ncellout are its layers.
+    With in_ptr / out_ptr (device addresses of the [n_rows, n_cols] float64 DEM and of a [3, n_rows, n_cols] float64
+    array that receives Au, e.g. torch tensors' data_ptr()) and shape = (n_rows, n_cols), everything stays in HBM
+    (filled_ptr: optional [n_rows, n_cols] float64 for the filled DEM) and only the two counters are returned.
+    """
+    cin = _abi.SplashUpslopeIn()
+    cin.min_slope_deg = float(min_slope_deg)
+    return _upslope_au("splash_upslope_area_run", cin, _abi.SplashUpslopeOut(), ("fill_sweeps", "accum_rounds"),
+                       {"filled": (return_filled, filled_ptr)}, elev, ymax, xres, yres, lonlat, ctx, in_ptr, out_ptr, shape)
+
+
+def upslope_areav2(elev, ymax: float, xres: float, yres: float, lonlat: bool = True, ctx: Context | None = None,
+                   return_filled: bool = False, return_angle: bool = False, in_ptr: int | None = None,
+                   out_ptr: int | None = None, filled_ptr: int | None = None, angle_ptr: int | None = None,
+                   shape: tuple | None = None) -> dict:
+    """upslope_areav2() of the reference (R/upslope_area.R:59-137, the branch for coarse or large grids that calls
+    TauDEM): pit removal to flat, D-infinity flow directions with flats resolved (Garbrecht and Martz), and the
+    D-infinity contributing area (see include/splash_cuda.h, splash_upslope_dinf_run, PARITY UNPINNED); with the in /
+    out neighbour counts of splash_terrain_run.
+
+    Arguments and results as upslope_area (no min_slope_deg: the fill is to flat), plus the counter flat_rounds and,
+    with return_angle (or angle_ptr on the device path), `angle`: the flow angle in radians counter-clockwise from
+    east in [0, 2 pi), NaN where a cell has no direction (NA cells, boundary cells).
+    """
+    return _upslope_au("splash_upslope_dinf_run", _abi.SplashDinfIn(), _abi.SplashDinfOut(),
+                       ("fill_sweeps", "flat_rounds", "accum_rounds"),
+                       {"filled": (return_filled, filled_ptr), "angle": (return_angle, angle_ptr)},
+                       elev, ymax, xres, yres, lonlat, ctx, in_ptr, out_ptr, shape)
 
 
 def month_starts(time_index_month, time_index) -> np.ndarray:

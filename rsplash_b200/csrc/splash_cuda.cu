@@ -2192,15 +2192,16 @@ int splash_terrain_run(splash_ctx* ctx, const splash_terrain_in* in, splash_terr
 
 // Per-row metrics of the upslope area (splash_upslope.cuh: UR_*), on the host with libm so that the kernels and a
 // numpy restatement (Python's math module is the same libm) share every operand.  No contraction into FMA.
-__attribute__((optimize("fp-contract=off"))) static void upslope_rows(const splash_upslope_in* in, std::vector<double>& rows) {
+__attribute__((optimize("fp-contract=off"))) static void upslope_rows(int64_t n_rows, double ymax, double xres, double yres,
+                                                                      int lonlat, double min_slope_deg, std::vector<double>& rows) {
     using namespace upslope;
-    const double t = tan(in->min_slope_deg * kpir);
-    rows.resize((size_t)in->n_rows * UR_N);
-    for (int64_t r = 0; r < in->n_rows; ++r) {
+    const double t = tan(min_slope_deg * kpir);
+    rows.resize((size_t)n_rows * UR_N);
+    for (int64_t r = 0; r < n_rows; ++r) {
         double* m = rows.data() + r * UR_N;
-        const double lat_c = in->ymax - ((double)r + 0.5) * in->yres;
-        const double dy = in->lonlat ? kEarthR * (in->yres * kpir) : in->yres;
-        const double dx = in->lonlat ? kEarthR * cos(lat_c * kpir) * (in->xres * kpir) : in->xres;
+        const double lat_c = ymax - ((double)r + 0.5) * yres;
+        const double dy = lonlat ? kEarthR * (yres * kpir) : yres;
+        const double dx = lonlat ? kEarthR * cos(lat_c * kpir) * (xres * kpir) : xres;
         const double dd = sqrt(dx * dx + dy * dy);
         const double rl = sqrt(dx * dy);
         m[UR_DX] = dx;
@@ -2212,7 +2213,169 @@ __attribute__((optimize("fp-contract=off"))) static void upslope_rows(const spla
         m[UR_EX] = dx * t;
         m[UR_EY] = dy * t;
         m[UR_ED] = dd * t;
+        m[UR_TX] = atan2(dy, dx);
+        m[UR_TY] = atan2(dx, dy);
     }
+}
+
+// The DEM geometry both upslope entry points take (splash_upslope_in / splash_dinf_in).
+struct UpslopeGeom {
+    int64_t n_rows, n_cols;
+    const double* elev;
+    double ymax, xres, yres;
+    int32_t lonlat, mem_kind;
+};
+
+static int upslope_check(splash_ctx* ctx, const UpslopeGeom& g) {
+    if (g.n_rows < 0 || g.n_cols < 0 || g.n_rows > (int64_t)upslope::kFT * 65535 || (g.n_cols > 0 && g.n_rows > INT32_MAX / g.n_cols))
+        return fail(ctx, SPLASH_ERR_BAD_ARG, "bad n_rows/n_cols (n_rows*n_cols must fit in int32, n_rows <= %d)", upslope::kFT * 65535);
+    if (g.mem_kind != SPLASH_MEM_HOST && g.mem_kind != SPLASH_MEM_DEVICE)
+        return fail(ctx, SPLASH_ERR_BAD_ARG, "mem_kind must be SPLASH_MEM_HOST or SPLASH_MEM_DEVICE");
+    if (!(g.xres > 0) || !(g.yres > 0) || !std::isfinite(g.xres) || !std::isfinite(g.yres))
+        return fail(ctx, SPLASH_ERR_BAD_ARG, "xres and yres must be positive and finite");
+    if (g.lonlat && !(g.ymax <= 90.0 && g.ymax - (double)g.n_rows * g.yres >= -90.0))
+        return fail(ctx, SPLASH_ERR_BAD_ARG, "lonlat: the rows must lie between -90 and 90 degrees");
+    return SPLASH_OK;
+}
+
+constexpr int kUpslopeBatch = 64;  // sweeps launched between two reads of their flags
+
+// The temporaries of one upslope call (freed on every return path) and the device views of its DEM and area.
+struct UpslopeRun {
+    const char* fn;
+    cudaStream_t S;
+    int64_t n;
+    bool host;
+    std::vector<double> rows;
+    TmpDev t_z, t_w0, t_w1, t_area, t_rows, t_ctl;
+    const double* z = nullptr;
+    const double* d_rows = nullptr;
+    double* area = nullptr;
+    double* w[2] = {nullptr, nullptr};
+    int* ctl = nullptr;    // upslope::AC_* control words
+    int* flags = nullptr;  // flags[0]: "the sweep before this batch changed something"; flags[1..batch]: the batch
+    int hctl[upslope::AC_N + 1 + kUpslopeBatch];
+};
+
+// Device buffers, per-row metrics, W's initial state; +-inf elevations are rejected here.
+static int upslope_begin(splash_ctx* ctx, UpslopeRun& u, const UpslopeGeom& g, double min_slope_deg, double* out_area) {
+    using namespace upslope;
+    CU(cudaSetDevice(ctx->device));
+    u.S = ctx->s_run[0];
+    u.n = g.n_rows * g.n_cols;
+    u.host = g.mem_kind == SPLASH_MEM_HOST;
+    upslope_rows(g.n_rows, g.ymax, g.xres, g.yres, g.lonlat, min_slope_deg, u.rows);
+    const size_t nb = (size_t)u.n * 8;
+    if (u.host) {
+        CU(cudaMalloc(&u.t_z.p, nb));
+        CU(cudaMalloc(&u.t_area.p, nb));
+        CU(cudaMemcpyAsync(u.t_z.p, g.elev, nb, cudaMemcpyHostToDevice, u.S));
+    }
+    CU(cudaMalloc(&u.t_w0.p, nb));
+    CU(cudaMalloc(&u.t_w1.p, nb));
+    CU(cudaMalloc(&u.t_rows.p, u.rows.size() * 8));
+    CU(cudaMalloc(&u.t_ctl.p, (AC_N + 1 + kUpslopeBatch) * sizeof(int)));
+    CU(cudaMemcpyAsync(u.t_rows.p, u.rows.data(), u.rows.size() * 8, cudaMemcpyHostToDevice, u.S));
+    u.ctl = (int*)u.t_ctl.p;
+    u.flags = u.ctl + AC_N;
+    CU(cudaMemsetAsync(u.ctl, 0, AC_N * sizeof(int), u.S));
+    u.z = u.host ? (const double*)u.t_z.p : g.elev;
+    u.d_rows = (const double*)u.t_rows.p;
+    u.area = u.host ? (double*)u.t_area.p : out_area;
+    u.w[0] = (double*)u.t_w0.p;
+    u.w[1] = (double*)u.t_w1.p;
+    FillParams fp{u.z, u.d_rows, (int)g.n_rows, (int)g.n_cols};
+    k_fill_init<<<(unsigned)((u.n + 255) / 256), 256, 0, u.S>>>(fp, u.w[0], u.ctl + AC_BADZ, u.ctl + AC_NVALID);
+    CU(cudaGetLastError());
+    CU(cudaMemcpyAsync(u.hctl, u.ctl, AC_N * sizeof(int), cudaMemcpyDeviceToHost, u.S));
+    CU(cudaStreamSynchronize(u.S));
+    if (u.hctl[AC_BADZ]) return fail(ctx, SPLASH_ERR_BAD_ARG, "%s: elev has +-inf values (NaN is NA)", u.fn);
+    return SPLASH_OK;
+}
+
+extern "C++" {  // templates inside the file's extern "C" block
+// Jacobi sweeps launched in batches between reads of their changed flags (no host round trip per sweep), until a
+// sweep changes nothing; at most n sweeps.  launch(j, s) enqueues global sweep s as sweep j of the batch.
+template <class Launch>
+static int run_sweeps(splash_ctx* ctx, UpslopeRun& u, const char* what, Launch launch, int64_t* sweeps_out) {
+    int64_t sweeps = 0;
+    bool converged = false;
+    for (int batch = 4; !converged;) {
+        const int one = 1;
+        CU(cudaMemcpyAsync(u.flags, &one, sizeof(int), cudaMemcpyHostToDevice, u.S));
+        CU(cudaMemsetAsync(u.flags + 1, 0, batch * sizeof(int), u.S));
+        for (int j = 1; j <= batch; ++j) launch(j, sweeps + j - 1);
+        CU(cudaGetLastError());
+        CU(cudaMemcpyAsync(u.hctl, u.flags + 1, batch * sizeof(int), cudaMemcpyDeviceToHost, u.S));
+        CU(cudaStreamSynchronize(u.S));
+        for (int j = 0; j < batch && !converged; ++j) {
+            ++sweeps;
+            converged = u.hctl[j] == 0;
+        }
+        if (!converged && sweeps >= u.n)
+            return fail(ctx, SPLASH_ERR_CUDA, "%s: %s did not converge in %lld sweeps", u.fn, what, (long long)u.n);
+        batch = std::min(2 * batch, kUpslopeBatch);
+    }
+    *sweeps_out = sweeps;
+    return SPLASH_OK;
+}
+
+// The fill; *wf: the filled surface (written by the last sweep, equal to its input: nothing changed).
+static int upslope_fill(splash_ctx* ctx, UpslopeRun& u, int n_rows, int n_cols, int64_t* sweeps, const double** wf) {
+    using namespace upslope;
+    FillParams fp{u.z, u.d_rows, n_rows, n_cols};
+    const dim3 fgrid((unsigned)((n_cols + kFT - 1) / kFT), (unsigned)((n_rows + kFT - 1) / kFT)), fblock(kFT, kFRows);
+    const int rc = run_sweeps(ctx, u, "the fill", [&](int j, int64_t s) {
+        k_fill_sweep<<<fgrid, fblock, 0, u.S>>>(fp, u.w[s & 1], u.w[(s + 1) & 1], u.flags, j);
+    }, sweeps);
+    if (rc) return rc;
+    *wf = u.w[*sweeps & 1];
+    return SPLASH_OK;
+}
+
+// Clear the frontier words of ctl before a seed kernel fills the first frontier (n_valid stays).
+static int rounds_reset(splash_ctx* ctx, UpslopeRun& u) {
+    CU(cudaMemsetAsync(u.ctl, 0, upslope::AC_NVALID * sizeof(int), u.S));
+    return SPLASH_OK;
+}
+
+// The frontier rounds of k_accum<Rule> in cooperative launches until the frontier is empty; a launch that does not
+// finish runs at least one round, and there are at most n rounds.
+template <class Rule>
+static int run_rounds(splash_ctx* ctx, UpslopeRun& u, Rule p, const char* what, int64_t* rounds) {
+    using namespace upslope;
+    int per_sm = 0;
+    CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_accum<Rule>, kAccThreads, 0));
+    if (per_sm < 1) return fail(ctx, SPLASH_ERR_CUDA, "%s: k_accum does not fit an SM", u.fn);
+    const unsigned agrid = (unsigned)std::max<int64_t>(1, std::min<int64_t>((int64_t)per_sm * ctx->sm_count, (u.n + kAccThreads - 1) / kAccThreads));
+    void* args[] = {&p};
+    int64_t launches = 0;
+    for (int batch = 2;; batch = std::min(2 * batch, 16)) {
+        if (launches > u.n + 1) return fail(ctx, SPLASH_ERR_CUDA, "%s: the %s did not finish", u.fn, what);
+        for (int j = 0; j < batch; ++j) CU(cudaLaunchCooperativeKernel((const void*)k_accum<Rule>, agrid, kAccThreads, args, 0, u.S));
+        launches += batch;
+        CU(cudaMemcpyAsync(u.hctl, u.ctl, AC_N * sizeof(int), cudaMemcpyDeviceToHost, u.S));
+        CU(cudaStreamSynchronize(u.S));
+        if (u.hctl[AC_ERR]) return fail(ctx, SPLASH_ERR_CUDA, "%s: more %s rounds than valid cells", u.fn, what);
+        if (u.hctl[AC_DONE]) break;
+    }
+    *rounds = u.hctl[AC_ROUNDS];
+    return SPLASH_OK;
+}
+
+}  // extern "C++"
+
+// area (and the optional filled surface) to the caller's arrays, then wait for the stream.
+static int upslope_finish(splash_ctx* ctx, UpslopeRun& u, double* area, double* filled, const double* wf) {
+    const size_t nb = (size_t)u.n * 8;
+    if (u.host) {
+        CU(cudaMemcpyAsync(area, u.area, nb, cudaMemcpyDeviceToHost, u.S));
+        if (filled) CU(cudaMemcpyAsync(filled, wf, nb, cudaMemcpyDeviceToHost, u.S));
+    } else if (filled) {
+        CU(cudaMemcpyAsync(filled, wf, nb, cudaMemcpyDeviceToDevice, u.S));
+    }
+    CU(cudaStreamSynchronize(u.S));
+    return SPLASH_OK;
 }
 
 int splash_upslope_area_run(splash_ctx* ctx, const splash_upslope_in* in, splash_upslope_out* out) {
@@ -2228,122 +2391,119 @@ int splash_upslope_area_run(splash_ctx* ctx, const splash_upslope_in* in, splash
     if (!in || !out) return fail(ctx, SPLASH_ERR_BAD_ARG, "splash_upslope_area_run: NULL in/out");
     out->fill_sweeps = 0;
     out->accum_rounds = 0;
-    const int64_t nr = in->n_rows, ncol = in->n_cols;
-    if (nr < 0 || ncol < 0 || nr > (int64_t)kFT * 65535 || (ncol > 0 && nr > INT32_MAX / ncol))
-        return fail(ctx, SPLASH_ERR_BAD_ARG, "bad n_rows/n_cols (n_rows*n_cols must fit in int32, n_rows <= %d)", kFT * 65535);
-    if (in->mem_kind != SPLASH_MEM_HOST && in->mem_kind != SPLASH_MEM_DEVICE)
-        return fail(ctx, SPLASH_ERR_BAD_ARG, "mem_kind must be SPLASH_MEM_HOST or SPLASH_MEM_DEVICE");
-    if (!(in->xres > 0) || !(in->yres > 0) || !std::isfinite(in->xres) || !std::isfinite(in->yres))
-        return fail(ctx, SPLASH_ERR_BAD_ARG, "xres and yres must be positive and finite");
+    UpslopeRun u;
+    u.fn = "splash_upslope_area_run";
+    const UpslopeGeom g{in->n_rows, in->n_cols, in->elev, in->ymax, in->xres, in->yres, in->lonlat, in->mem_kind};
+    if (int rc = upslope_check(ctx, g)) return rc;
     if (!std::isfinite(in->min_slope_deg) || !(in->min_slope_deg > 0.0) || !(in->min_slope_deg < 90.0))
         return fail(ctx, SPLASH_ERR_BAD_ARG, "min_slope_deg must be in (0, 90)");
-    if (in->lonlat && !(in->ymax <= 90.0 && in->ymax - (double)nr * in->yres >= -90.0))
-        return fail(ctx, SPLASH_ERR_BAD_ARG, "lonlat: the rows must lie between -90 and 90 degrees");
-    const int64_t n = nr * ncol;
-    if (n == 0) return SPLASH_OK;
+    const int nr = (int)in->n_rows, ncol = (int)in->n_cols;
+    if ((int64_t)nr * ncol == 0) return SPLASH_OK;
     if (!in->elev || !out->area) return fail(ctx, SPLASH_ERR_BAD_ARG, "NULL elev/area");
-    CU(cudaSetDevice(ctx->device));
-    cudaStream_t S = ctx->s_run[0];
-    std::vector<double> rows;
-    upslope_rows(in, rows);
-    const size_t nb = (size_t)n * 8;
-    TmpDev t_z, t_w0, t_w1, t_s, t_area, t_ndon, t_f0, t_f1, t_rows, t_ctl;  // freed on every return path
-    const bool host = in->mem_kind == SPLASH_MEM_HOST;
-    if (host) {
-        CU(cudaMalloc(&t_z.p, nb));
-        CU(cudaMalloc(&t_area.p, nb));
-        CU(cudaMemcpyAsync(t_z.p, in->elev, nb, cudaMemcpyHostToDevice, S));
-    }
-    CU(cudaMalloc(&t_w0.p, nb));
-    CU(cudaMalloc(&t_w1.p, nb));
-    CU(cudaMalloc(&t_s.p, nb));
-    CU(cudaMalloc(&t_ndon.p, (size_t)n * 4));
-    CU(cudaMalloc(&t_f0.p, (size_t)n * 4));
-    CU(cudaMalloc(&t_f1.p, (size_t)n * 4));
-    CU(cudaMalloc(&t_rows.p, rows.size() * 8));
-    constexpr int kMaxBatch = 64;  // fill sweeps launched between two reads of their flags
-    CU(cudaMalloc(&t_ctl.p, (AC_N + 1 + kMaxBatch) * sizeof(int)));
-    CU(cudaMemcpyAsync(t_rows.p, rows.data(), rows.size() * 8, cudaMemcpyHostToDevice, S));
-    int* ctl = (int*)t_ctl.p;
-    int* flags = ctl + AC_N;  // flags[0]: "the sweep before this batch changed something"; flags[1..batch]: the batch
-    CU(cudaMemsetAsync(ctl, 0, AC_N * sizeof(int), S));
-    const double* z = host ? (const double*)t_z.p : in->elev;
-    double* area = host ? (double*)t_area.p : out->area;
-    double* w[2] = {(double*)t_w0.p, (double*)t_w1.p};
-    FillParams fp{z, (const double*)t_rows.p, (int)nr, (int)ncol};
-    const unsigned grid = (unsigned)((n + 255) / 256);
-    k_fill_init<<<grid, 256, 0, S>>>(fp, w[0], ctl + AC_BADZ, ctl + AC_NVALID);
-    CU(cudaGetLastError());
-    int hctl[AC_N + 1 + kMaxBatch];
-    CU(cudaMemcpyAsync(hctl, ctl, AC_N * sizeof(int), cudaMemcpyDeviceToHost, S));
-    CU(cudaStreamSynchronize(S));
-    if (hctl[AC_BADZ]) return fail(ctx, SPLASH_ERR_BAD_ARG, "splash_upslope_area_run: elev has +-inf values (NaN is NA)");
-
-    // fill: batches of sweeps between reads of the flags (no host round trip per sweep); bound n sweeps
-    const dim3 fgrid((unsigned)((ncol + kFT - 1) / kFT), (unsigned)((nr + kFT - 1) / kFT)), fblock(kFT, kFRows);
-    int64_t sweeps = 0;
-    bool converged = false;
-    for (int batch = 4; !converged;) {
-        const int one = 1;
-        CU(cudaMemcpyAsync(flags, &one, sizeof(int), cudaMemcpyHostToDevice, S));
-        CU(cudaMemsetAsync(flags + 1, 0, batch * sizeof(int), S));
-        for (int j = 1; j <= batch; ++j) {
-            const int64_t s = sweeps + j - 1;
-            k_fill_sweep<<<fgrid, fblock, 0, S>>>(fp, w[s & 1], w[(s + 1) & 1], flags, j);
-        }
-        CU(cudaGetLastError());
-        CU(cudaMemcpyAsync(hctl, flags + 1, batch * sizeof(int), cudaMemcpyDeviceToHost, S));
-        CU(cudaStreamSynchronize(S));
-        for (int j = 0; j < batch && !converged; ++j) {
-            ++sweeps;
-            converged = hctl[j] == 0;
-        }
-        if (!converged && sweeps >= n)
-            return fail(ctx, SPLASH_ERR_CUDA, "splash_upslope_area_run: the fill did not converge in %lld sweeps", (long long)n);
-        batch = std::min(2 * batch, kMaxBatch);
-    }
-    out->fill_sweeps = sweeps;
-    const double* wf = w[sweeps & 1];  // written by the last sweep (equal to its input: nothing changed)
+    if (int rc = upslope_begin(ctx, u, g, in->min_slope_deg, out->area)) return rc;
+    const double* wf = nullptr;
+    if (int rc = upslope_fill(ctx, u, nr, ncol, &out->fill_sweeps, &wf)) return rc;
 
     // accumulation
-    AccumParams ap{};
+    TmpDev t_s, t_ndon, t_f0, t_f1;
+    CU(cudaMalloc(&t_s.p, (size_t)u.n * 8));
+    CU(cudaMalloc(&t_ndon.p, (size_t)u.n * 4));
+    CU(cudaMalloc(&t_f0.p, (size_t)u.n * 4));
+    CU(cudaMalloc(&t_f1.p, (size_t)u.n * 4));
+    MfdRule ap{};
     ap.w = wf;
-    ap.rows = (const double*)t_rows.p;
+    ap.rows = u.d_rows;
     ap.s = (double*)t_s.p;
-    ap.area = area;
+    ap.area = u.area;
     ap.ndon = (int*)t_ndon.p;
     ap.front[0] = (int*)t_f0.p;
     ap.front[1] = (int*)t_f1.p;
-    ap.ctl = ctl;
-    ap.n_rows = (int)nr;
-    ap.n_cols = (int)ncol;
-    k_flow_prep<<<grid, 256, 0, S>>>(ap);
+    ap.ctl = u.ctl;
+    ap.n_rows = nr;
+    ap.n_cols = ncol;
+    if (int rc = rounds_reset(ctx, u)) return rc;
+    k_flow_prep<<<(unsigned)((u.n + 255) / 256), 256, 0, u.S>>>(ap);
     CU(cudaGetLastError());
-    int per_sm = 0;
-    CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_accum, kAccThreads, 0));
-    if (per_sm < 1) return fail(ctx, SPLASH_ERR_CUDA, "splash_upslope_area_run: k_accum does not fit an SM");
-    const unsigned agrid = (unsigned)std::max<int64_t>(1, std::min<int64_t>((int64_t)per_sm * ctx->sm_count, (n + kAccThreads - 1) / kAccThreads));
-    void* args[] = {&ap};
-    // a launch that does not finish runs at least one round, and there are at most n rounds
-    int64_t launches = 0;
-    for (int batch = 2;; batch = std::min(2 * batch, 16)) {
-        if (launches > n + 1) return fail(ctx, SPLASH_ERR_CUDA, "splash_upslope_area_run: the accumulation did not finish");
-        for (int j = 0; j < batch; ++j) CU(cudaLaunchCooperativeKernel((const void*)k_accum, agrid, kAccThreads, args, 0, S));
-        launches += batch;
-        CU(cudaMemcpyAsync(hctl, ctl, AC_N * sizeof(int), cudaMemcpyDeviceToHost, S));
-        CU(cudaStreamSynchronize(S));
-        if (hctl[AC_ERR]) return fail(ctx, SPLASH_ERR_CUDA, "splash_upslope_area_run: more accumulation rounds than valid cells");
-        if (hctl[AC_DONE]) break;
+    if (int rc = run_rounds(ctx, u, ap, "accumulation", &out->accum_rounds)) return rc;
+    return upslope_finish(ctx, u, out->area, out->filled, wf);
+}
+
+int splash_upslope_dinf_run(splash_ctx* ctx, const splash_dinf_in* in, splash_dinf_out* out) {
+    using namespace upslope;
+    if (ctx && ctx->multi) {  // single-GPU work: the context's first lane does it
+        splash_ctx* lane = first_lane(ctx);
+        const int rc = splash_upslope_dinf_run(lane, in, out);
+        ctx->err = lane->err;
+        return rc;
     }
-    out->accum_rounds = hctl[AC_ROUNDS];
-    if (host) {
-        CU(cudaMemcpyAsync(out->area, area, nb, cudaMemcpyDeviceToHost, S));
-        if (out->filled) CU(cudaMemcpyAsync(out->filled, wf, nb, cudaMemcpyDeviceToHost, S));
-    } else if (out->filled) {
-        CU(cudaMemcpyAsync(out->filled, wf, nb, cudaMemcpyDeviceToDevice, S));
+    if (!ctx) return SPLASH_ERR_BAD_ARG;
+    ctx->err.clear();
+    if (!in || !out) return fail(ctx, SPLASH_ERR_BAD_ARG, "splash_upslope_dinf_run: NULL in/out");
+    out->fill_sweeps = 0;
+    out->flat_rounds = 0;
+    out->accum_rounds = 0;
+    UpslopeRun u;
+    u.fn = "splash_upslope_dinf_run";
+    const UpslopeGeom g{in->n_rows, in->n_cols, in->elev, in->ymax, in->xres, in->yres, in->lonlat, in->mem_kind};
+    if (int rc = upslope_check(ctx, g)) return rc;
+    const int nr = (int)in->n_rows, ncol = (int)in->n_cols;
+    if ((int64_t)nr * ncol == 0) return SPLASH_OK;
+    if (!in->elev || !out->area) return fail(ctx, SPLASH_ERR_BAD_ARG, "splash_upslope_dinf_run: NULL elev/area");
+    if (int rc = upslope_begin(ctx, u, g, 0.0, out->area)) return rc;  // eps = 0: PitRemove fills to flat
+    const double* wf = nullptr;
+    if (int rc = upslope_fill(ctx, u, nr, ncol, &out->fill_sweeps, &wf)) return rc;
+    const int64_t n = u.n;
+    const unsigned grid = (unsigned)((n + 255) / 256);
+
+    // flats: classes, labels, the two distances, the per-flat maximum, the mask M (in place of the towards distance)
+    TmpDev t_cls, t_lab0, t_lab1, t_tow, t_away, t_hmax, t_ndon, t_f0, t_f1, t_rec, t_pd, t_angle;
+    CU(cudaMalloc(&t_cls.p, (size_t)n));
+    for (TmpDev* t : {&t_lab0, &t_lab1, &t_tow, &t_away, &t_hmax, &t_ndon, &t_f0, &t_f1}) CU(cudaMalloc(&t->p, (size_t)n * 4));
+    CU(cudaMalloc(&t_rec.p, (size_t)n));
+    CU(cudaMalloc(&t_pd.p, (size_t)n * 8));
+    unsigned char* cls = (unsigned char*)t_cls.p;
+    int* lab[2] = {(int*)t_lab0.p, (int*)t_lab1.p};
+    int* front[2] = {(int*)t_f0.p, (int*)t_f1.p};
+    FlatParams fp{wf, cls, (int*)t_tow.p, (int*)t_away.p, (int*)t_hmax.p, nr, ncol};
+    k_flat_mark<<<grid, 256, 0, u.S>>>(fp, lab[0]);
+    CU(cudaGetLastError());
+    int64_t label_sweeps = 0, tow_rounds = 0, away_rounds = 0;
+    if (int rc = run_sweeps(ctx, u, "the flat labelling", [&](int j, int64_t s) {
+            k_flat_label<<<grid, 256, 0, u.S>>>(fp, lab[s & 1], lab[(s + 1) & 1], u.flags, j);
+        }, &label_sweeps))
+        return rc;
+    const int* label = lab[label_sweeps & 1];
+    if (int rc = rounds_reset(ctx, u)) return rc;
+    k_flat_seed<false><<<grid, 256, 0, u.S>>>(fp, front[0], u.ctl);
+    CU(cudaGetLastError());
+    if (int rc = run_rounds(ctx, u, FlatBfs{cls, fp.tow, {front[0], front[1]}, u.ctl, nr, ncol}, "flat distance", &tow_rounds)) return rc;
+    if (int rc = rounds_reset(ctx, u)) return rc;
+    k_flat_seed<true><<<grid, 256, 0, u.S>>>(fp, front[0], u.ctl);
+    CU(cudaGetLastError());
+    if (int rc = run_rounds(ctx, u, FlatBfs{cls, fp.away, {front[0], front[1]}, u.ctl, nr, ncol}, "flat distance", &away_rounds)) return rc;
+    k_flat_height<<<grid, 256, 0, u.S>>>(fp, label);
+    k_flat_mask<<<grid, 256, 0, u.S>>>(fp, label);
+    CU(cudaGetLastError());
+    out->flat_rounds = label_sweeps + tow_rounds + away_rounds;
+
+    // directions
+    double* angle = out->angle;
+    if (angle && u.host) {
+        CU(cudaMalloc(&t_angle.p, (size_t)n * 8));
+        angle = (double*)t_angle.p;
     }
-    CU(cudaStreamSynchronize(S));
-    return SPLASH_OK;
+    DinfParams dp{wf, u.d_rows, cls, fp.tow, (unsigned char*)t_rec.p, (double*)t_pd.p, angle, nr, ncol};
+    k_dinf_dir<<<grid, 256, 0, u.S>>>(dp);
+    CU(cudaGetLastError());
+
+    // accumulation
+    DinfRule ar{dp.rec, dp.pd, u.d_rows, u.area, (int*)t_ndon.p, {front[0], front[1]}, u.ctl, nr, ncol};
+    if (int rc = rounds_reset(ctx, u)) return rc;
+    k_dinf_prep<<<grid, 256, 0, u.S>>>(ar, wf);
+    CU(cudaGetLastError());
+    if (int rc = run_rounds(ctx, u, ar, "accumulation", &out->accum_rounds)) return rc;
+    if (out->angle && u.host) CU(cudaMemcpyAsync(out->angle, angle, (size_t)n * 8, cudaMemcpyDeviceToHost, u.S));
+    return upslope_finish(ctx, u, out->area, out->filled, wf);
 }
 
 int splash_month2day_linear(splash_ctx* ctx, const splash_m2d_in* in, void* daily_out) {
