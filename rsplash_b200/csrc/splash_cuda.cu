@@ -10,10 +10,10 @@
 //                     also day 1 of the next pass) with compaction, then days 2..365 of the survivors;
 //                     the list sizes stay on the device, the host never waits for them
 //   k_run_bulk        the run_all day loop of every cell whose spin-up is finished: 768 threads per SM, state in
-//                     registers, the state half's constants in shared memory and the forcing half's read from
-//                     the constant matrix (HybridCC), optionally in regime-sorted order (k_regime_*), next day's
+//                     registers, the state half's constants in shared memory and the forcing half's in tensor
+//                     memory (TmemCC), optionally in regime-sorted order (k_regime_*), next day's
 //                     forcing staged by cp.async, outputs written with streaming stores (daily) or reduced per
-//                     month in registers (monthly)
+//                     month in tensor memory (monthly)
 //   k_run_list        per-thread state machine (rest of the spin-up, then the day loop) for the few cells
 //                     that outlive the lock-step passes; lanes fetch cells from a device-side queue
 //   k_pool_*          move those stragglers (constants, state, forcing columns) into a context-wide
@@ -103,9 +103,6 @@ constexpr int kUBound = kUThreads + SPLASH_UREG_SLACK;
 #ifndef SPLASH_BULK_REGS
 #define SPLASH_BULK_REGS (SPLASH_BULK_THREADS > 512 ? 80 : 104)
 #endif
-#ifndef SPLASH_BULK_RELOAD
-#define SPLASH_BULK_RELOAD 1
-#endif
 #define SPLASH_BULK_BOUNDS __maxnreg__(SPLASH_BULK_REGS)
 #if SPLASH_UREGS > 0
 #define SPLASH_UNIFORM_BOUNDS __maxnreg__(SPLASH_UREGS)
@@ -145,39 +142,152 @@ struct StridedCC {  // column of a [NCC][stride] matrix (shared or global memory
 
 // Shapes of the uniform kernels.  The day step keeps 52 constants per cell; as private shared-memory columns they cap a
 // CTA at 512 cells (213 KB), i.e. four warps per scheduler -- too few to hide the FP64 dependency latency (ncu r02:
-// 3.6 cycles of fixed-latency wait per issued instruction).  A kernel compiled for more than 512 threads keeps only the
-// constants of the state half (the dependent chain) in shared memory and reads the 18 that the forcing half and the
-// output stage use -- state-independent, so their loads are issued at the top of the day and are not waited for until
-// the forcing half needs them -- from the constant matrix in global memory (L2 hits: 15 MB for the whole device).
+// 3.6 cycles of fixed-latency wait per issued instruction).  A bulk launch of more than 512 threads keeps only the
+// constants of the state half (the dependent chain) in shared memory and the 18 that the forcing half and the output
+// stage use in the thread's tensor-memory columns (TmemCC), from where each section of the day step loads its group.
 // The bulk launch runs 768 threads x 80 registers = six warps per scheduler (+8 % on the kernel alone, measured; the
 // spin-up kernels keep 512 threads: their late rounds are short lists, where larger CTAs were measured slower).
 constexpr int kBThreads = SPLASH_BULK_THREADS;
 template <int NT> __host__ __device__ constexpr bool hybrid_cc() { return NT > 512; }
 
-// constants that only day_forcing (and the output stage) read
-__host__ __device__ constexpr bool cc_cold(int k) {
-    return k == C_ELEV_K || k == C_LAT_K || k == C_TT || k == C_COS_LAT || k == C_SIN_LAT || k == C_SIN_S || k == C_COS_S ||
-           k == C_COS_A || k == C_SIN_A || k == C_TAU_O || k == C_TAU_A || k == C_PATM || k == C_PBAR || k == C_PBARF ||
-           k == C_VISC0 || k == C_INTPERM || k == C_INV_TAU_B || k == C_WRR;
+// Constants that only day_forcing (and the output stage) read, with their slots, the order of their tensor-memory columns
+// (below): each cc_fetch group is a contiguous run of slots.  -1: a hot constant.
+constexpr int kNCold = 18;
+__host__ __device__ constexpr int cc_cold_slot(int k) {
+    switch (k) {
+        case C_COS_LAT: return 0;  // CCG_GEOMETRY: slots 0..8
+        case C_SIN_LAT: return 1;
+        case C_SIN_S: return 2;
+        case C_COS_S: return 3;
+        case C_COS_A: return 4;
+        case C_SIN_A: return 5;
+        case C_TAU_O: return 6;
+        case C_TAU_A: return 7;
+        case C_INV_TAU_B: return 8;
+        case C_WRR: return 9;  // CCG_OUTPUT
+        case C_ELEV_K: return 10;  // CCG_SNOW: 10..12
+        case C_LAT_K: return 11;
+        case C_TT: return 12;
+        case C_PATM: return 13;  // CCG_PRESSURE: 13..17
+        case C_PBAR: return 14;
+        case C_PBARF: return 15;
+        case C_VISC0: return 16;
+        case C_INTPERM: return 17;
+        default: return -1;
+    }
 }
+__host__ __device__ constexpr bool cc_cold(int k) { return cc_cold_slot(k) >= 0; }
 __host__ __device__ constexpr int cc_hot_slot(int k) {  // rank of constant k among the hot ones
     int n = 0;
     for (int j = 0; j < k; ++j) n += cc_cold(j) ? 0 : 1;
     return n;
 }
 constexpr int kHotCC = cc_hot_slot(NCC_DAY);
-static_assert(kHotCC + 18 == NCC_DAY && cc_hot_slot(0) == 0 && !cc_cold(C_RES) && cc_cold(C_WRR) && cc_cold(C_TT),
-              "hot / cold split of the day step's constants");
+static_assert(kNCold == 18 && kHotCC + kNCold == NCC_DAY && cc_hot_slot(0) == 0 && !cc_cold(C_RES) && cc_cold(C_WRR) &&
+              cc_cold(C_TT), "hot / cold split of the day step's constants");
+
+// ---------------------------------------------------------------------------------------------
+// tensor memory (TMEM) as private per-thread storage of the bulk launch
+// ---------------------------------------------------------------------------------------------
+// The bulk CTA allocates all 512 columns of its SM's TMEM (its shared memory keeps any second bulk CTA off the SM, so the
+// allocation never waits, static_assert at bulk_smem).  tcgen05.ld / st of the 32x32b shape move a warp's registers to
+// and from the 32 TMEM lanes of its quadrant (warp % 4), one lane per thread; each warp owns the columns
+// [(warp / 4) * kTmemSlice, + kTmemSlice) of its lanes.  Columns of a thread's slice:
+//   0..35   the cold constants in cc_cold_slot order, two 32-bit columns per double (low word first)
+//   36..37  the month's sum of layer 8, 40..42 its three counts, 48..63 the sums of layers 0..7 (monthly launch)
+// Every load and store is a power-of-two column count at a column aligned to it.  The instructions are warp-collective
+// (.sync.aligned): every lane of a warp executes each of them, converged.
+constexpr int kTmemCols = 512;
+constexpr int kTmemSlice = 64;
+constexpr int kTmemAcc = 48, kTmemAcc8 = 36, kTmemCnt = 40;
+static_assert(2 * kNCold <= kTmemAcc8, "TMEM column map");
+
+template <int N> __device__ __forceinline__ void tmem_ld(uint32_t ta, uint32_t* r);
+template <> __device__ __forceinline__ void tmem_ld<2>(uint32_t ta, uint32_t* r) {
+    asm volatile("tcgen05.ld.sync.aligned.32x32b.x2.b32 {%0, %1}, [%2];" : "=r"(r[0]), "=r"(r[1]) : "r"(ta));
+}
+template <> __device__ __forceinline__ void tmem_ld<4>(uint32_t ta, uint32_t* r) {
+    asm volatile("tcgen05.ld.sync.aligned.32x32b.x4.b32 {%0, %1, %2, %3}, [%4];"
+                 : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]) : "r"(ta));
+}
+template <> __device__ __forceinline__ void tmem_ld<8>(uint32_t ta, uint32_t* r) {
+    asm volatile("tcgen05.ld.sync.aligned.32x32b.x8.b32 {%0, %1, %2, %3, %4, %5, %6, %7}, [%8];"
+                 : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]) : "r"(ta));
+}
+template <> __device__ __forceinline__ void tmem_ld<16>(uint32_t ta, uint32_t* r) {
+    asm volatile("tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15}, [%16];"
+                 : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]),
+                   "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15])
+                 : "r"(ta));
+}
+template <int N> __device__ __forceinline__ void tmem_st(uint32_t ta, const uint32_t* r);
+template <> __device__ __forceinline__ void tmem_st<2>(uint32_t ta, const uint32_t* r) {
+    asm volatile("tcgen05.st.sync.aligned.32x32b.x2.b32 [%0], {%1, %2};" ::"r"(ta), "r"(r[0]), "r"(r[1]));
+}
+template <> __device__ __forceinline__ void tmem_st<4>(uint32_t ta, const uint32_t* r) {
+    asm volatile("tcgen05.st.sync.aligned.32x32b.x4.b32 [%0], {%1, %2, %3, %4};" ::"r"(ta), "r"(r[0]), "r"(r[1]), "r"(r[2]),
+                 "r"(r[3]));
+}
+template <> __device__ __forceinline__ void tmem_st<16>(uint32_t ta, const uint32_t* r) {
+    asm volatile("tcgen05.st.sync.aligned.32x32b.x16.b32 [%0], {%1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, %16};"
+                 ::"r"(ta), "r"(r[0]), "r"(r[1]), "r"(r[2]), "r"(r[3]), "r"(r[4]), "r"(r[5]), "r"(r[6]), "r"(r[7]), "r"(r[8]),
+                   "r"(r[9]), "r"(r[10]), "r"(r[11]), "r"(r[12]), "r"(r[13]), "r"(r[14]), "r"(r[15]));
+}
+// Waits for this thread's outstanding loads.  The loaded registers pass through an empty asm after the wait, so that no
+// use of them can be scheduled above it.
+__device__ __forceinline__ void tmem_wait_ld(uint32_t* r, int n) {
+    asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+#pragma unroll
+    for (int j = 0; j < n; ++j) asm volatile("" : "+r"(r[j]));
+}
+__device__ __forceinline__ void tmem_wait_st() { asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory"); }
+
+// Allocates the CTA's TMEM (warp 0) and publishes its address; returns this thread's column slice.  Every thread of the
+// CTA calls it, and every thread later calls tmem_close.
+__device__ __forceinline__ uint32_t tmem_open(uint32_t* s_base) {
+    const unsigned warp = threadIdx.x / 32;
+    if (warp == 0) {
+        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(
+                         (unsigned)__cvta_generic_to_shared(s_base)), "n"(kTmemCols));
+        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;");
+    }
+    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+    __syncthreads();
+    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+    return *(volatile uint32_t*)s_base + ((32u * (warp % 4)) << 16) + (warp / 4) * (uint32_t)kTmemSlice;
+}
+__device__ __forceinline__ void tmem_close(const uint32_t* s_base) {
+    tmem_wait_st();
+    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+    __syncthreads();
+    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+    if (threadIdx.x / 32 == 0)
+        asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(*(volatile const uint32_t*)s_base), "n"(kTmemCols));
+}
 
 template <int NT>
-struct HybridCC {  // read-only: hot constants from the thread's shared-memory column, cold ones from the global matrix
+struct TmemCC {  // read-only: hot constants from the thread's shared-memory column, cold ones from its TMEM columns
     const double* hot;
-    const double* cold;  // p.cc + c
-    int64_t gstride;
-    __device__ __forceinline__ double operator()(int k) const {
-        return cc_cold(k) ? __ldg(cold + (int64_t)k * gstride) : hot[cc_hot_slot(k) * NT];
+    uint32_t ta;
+    mutable double cold[kNCold];  // the groups cc_fetch brought into registers
+    __device__ __forceinline__ double operator()(int k) const { return cc_cold(k) ? cold[cc_cold_slot(k)] : hot[cc_hot_slot(k) * NT]; }
+    // slots [lo, hi) of group g: one or two loads, one wait
+    __device__ __forceinline__ void fetch(CCGroup g) const {
+        uint32_t r[2 * kNCold];
+        int lo, hi;
+        switch (g) {
+            case CCG_GEOMETRY: tmem_ld<16>(ta, r); tmem_ld<2>(ta + 16, r + 16); lo = 0; hi = 9; break;
+            case CCG_OUTPUT: tmem_ld<2>(ta + 18, r + 18); lo = 9; hi = 10; break;
+            case CCG_SNOW: tmem_ld<4>(ta + 20, r + 20); tmem_ld<2>(ta + 24, r + 24); lo = 10; hi = 13; break;
+            default: tmem_ld<2>(ta + 26, r + 26); tmem_ld<8>(ta + 28, r + 28); lo = 13; hi = 18; break;
+        }
+        tmem_wait_ld(r + 2 * lo, 2 * (hi - lo));
+#pragma unroll
+        for (int s = lo; s < hi; ++s) cold[s] = __hiloint2double(r[2 * s + 1], r[2 * s]);
     }
 };
+template <int NT>
+__device__ __forceinline__ void cc_fetch(const TmemCC<NT>& cc, CCGroup g) { cc.fetch(g); }
 
 template <typename T>
 __device__ __forceinline__ double ld_stream(const T* p) {
@@ -533,32 +643,49 @@ __device__ __forceinline__ bool spin_decide(const CellState& Ek, double chk_wn, 
     return cont;
 }
 
-// a uniform kernel's constants: all of them (StridedCC) or the hot ones (HybridCC) into the thread's shared-memory column
+// a uniform kernel's constants: all of them (StridedCC) into the thread's shared-memory column
 template <int NT>
 __device__ __forceinline__ void stage_cc(const RunParams& p, int c, bool live, double* s_cc, StridedCC& cc) {
     cc = StridedCC{s_cc + threadIdx.x, NT};
     if (live) load_cc(p, c, cc);
 }
+// the bulk launch's split: hot constants into the shared-memory column, cold ones into the thread's TMEM columns `ta`
 template <int NT>
-__device__ __forceinline__ void stage_cc(const RunParams& p, int c, bool live, double* s_cc, HybridCC<NT>& cc) {
-    cc = HybridCC<NT>{s_cc + threadIdx.x, p.cc + c, p.cpitch};
-    if (live) {
+__device__ __forceinline__ void stage_cc(const RunParams& p, int c, bool live, double* s_cc, uint32_t ta, TmemCC<NT>& cc) {
+    cc.hot = s_cc + threadIdx.x;
+    cc.ta = ta;
+    uint32_t r[2 * kNCold];
 #pragma unroll
-        for (int k = 0; k < NCC_DAY; ++k)
-            if (!cc_cold(k)) s_cc[cc_hot_slot(k) * NT + threadIdx.x] = p.cc[(int64_t)k * p.cpitch + c];
+    for (int k = 0; k < NCC_DAY; ++k) {
+        const double v = live ? p.cc[(int64_t)k * p.cpitch + c] : 0.0;
+        if (cc_cold(k)) {
+            r[2 * cc_cold_slot(k)] = (uint32_t)__double2loint(v);
+            r[2 * cc_cold_slot(k) + 1] = (uint32_t)__double2hiint(v);
+        } else {
+            s_cc[cc_hot_slot(k) * NT + threadIdx.x] = v;
+        }
     }
+    tmem_st<16>(ta, r);
+    tmem_st<16>(ta + 16, r + 16);
+    tmem_st<4>(ta + 32, r + 32);
 }
-template <int NT> using ShapeCC = std::conditional_t<hybrid_cc<NT>(), HybridCC<NT>, StridedCC>;
+template <int NT>
+__device__ __forceinline__ void stage_cc(const RunParams& p, int c, bool live, double* s_cc, uint32_t, StridedCC& cc) {
+    stage_cc<NT>(p, c, live, s_cc, cc);
+}
+template <int NT> using ShapeCC = std::conditional_t<hybrid_cc<NT>(), TmemCC<NT>, StridedCC>;
 template <int NT> __host__ __device__ constexpr int staged_cc() { return hybrid_cc<NT>() ? kHotCC : (int)NCC_DAY; }  // constants per cell in shared memory
+// the spin-up kernels keep all their constants in shared memory (52 x 512 x 8 B = 208 KB)
+static_assert(!hybrid_cc<kUThreads>(), "the uniform spin-up kernels run at most 512 threads per CTA");
 
 // lateral_consts on a uniform kernel's constants: the four results go to the thread's shared-memory column and to the
-// constant matrix (HybridCC is read-only, so the arithmetic runs on a scratch copy of the three inputs)
+// constant matrix (the arithmetic runs on a scratch copy of the three inputs)
 struct ScratchCC {
     double v[NCC];
     __device__ __forceinline__ double& operator()(int k) { return v[k]; }
 };
 template <int NT>
-__device__ __forceinline__ void apply_lateral(const RunParams& p, int c, double* s_cc, const ShapeCC<NT>& cc, double AI) {
+__device__ __forceinline__ void apply_lateral(const RunParams& p, int c, double* s_cc, const StridedCC& cc, double AI) {
     ScratchCC t;
     t(C_SIDOCT) = cc(C_SIDOCT);
     t(C_DEPTH) = cc(C_DEPTH);
@@ -568,7 +695,7 @@ __device__ __forceinline__ void apply_lateral(const RunParams& p, int c, double*
 #pragma unroll
     for (int j = 0; j < 4; ++j) {
         const int k = out[j];
-        s_cc[(hybrid_cc<NT>() ? cc_hot_slot(k) : k) * NT + threadIdx.x] = t(k);
+        s_cc[k * NT + threadIdx.x] = t(k);
         p.cc[(int64_t)k * p.cpitch + c] = t(k);
     }
 }
@@ -579,7 +706,7 @@ __global__ void SPLASH_UNIFORM_BOUNDS k_spin_first(RunParams p) {
     extern __shared__ double s_cc[];
     const int c = blockIdx.x * kUThreads + threadIdx.x;
     const bool live = c < p.n_cells;  // threads past the tile's end idle through the loop: every thread reaches every barrier
-    ShapeCC<kUThreads> cc;
+    StridedCC cc;
     stage_cc<kUThreads>(p, live ? c : 0, live, s_cc, cc);
     const double RES = live ? cc(C_RES) : 0.0;
     CellState st;
@@ -678,7 +805,7 @@ __global__ void SPLASH_UNIFORM_BOUNDS k_spin_rest(RunParams p) {
     const bool live = i < n_list;  // the list's last CTA: idle threads still reach every barrier
     const int c = live ? p.lists[(r + 1) & 1][i] : 0;
     SPLASH_CHECK(c >= 0 && c < p.n_cells && n_list <= (unsigned long long)p.n_cells, 103);
-    ShapeCC<kUThreads> cc;
+    StridedCC cc;
     stage_cc<kUThreads>(p, c, live, s_cc, cc);
     CellState st{};
     if (live) st = load_state(p.w, c);
@@ -722,11 +849,7 @@ __device__ __forceinline__ void emit_day(const RunParams& p, int c, int d, const
     if (sm_lim > 1) sm_lim = 1.0;
     const double v[9] = {st.wn, o.ro, o.pet, o.aet, st.snow, o.cond, o.bflow, o.netr, sm_lim};
     if (kMonthly) {
-#ifdef SPLASH_MACC_LOCAL  // experiment: a rolled loop keeps the nine sums in local memory instead of 18 registers
-#pragma unroll 1
-#else
 #pragma unroll
-#endif
         for (int k = 0; k < 9; ++k)
             if (!isnan(v[k])) m.acc[k] += v[k];
         if (!isnan(v[0])) ++m.cnt[0];
@@ -752,59 +875,111 @@ __device__ __forceinline__ void emit_day(const RunParams& p, int c, int d, const
     }
 }
 
+// the bulk launch's MonthAcc in the thread's TMEM columns (kTmemAcc, kTmemAcc8, kTmemCnt)
+__device__ __forceinline__ MonthAcc tmem_load_macc(uint32_t ta) {
+    uint32_t r[22];
+    tmem_ld<16>(ta + kTmemAcc, r);
+    tmem_ld<2>(ta + kTmemAcc8, r + 16);
+    tmem_ld<4>(ta + kTmemCnt, r + 18);
+    tmem_wait_ld(r, 21);
+    MonthAcc m;
+#pragma unroll
+    for (int k = 0; k < 9; ++k) m.acc[k] = __hiloint2double(r[2 * k + 1], r[2 * k]);
+#pragma unroll
+    for (int j = 0; j < 3; ++j) m.cnt[j] = (int)r[18 + j];
+    return m;
+}
+__device__ __forceinline__ void tmem_store_macc(uint32_t ta, const MonthAcc& m) {
+    uint32_t r[22];
+#pragma unroll
+    for (int k = 0; k < 9; ++k) {
+        r[2 * k] = (uint32_t)__double2loint(m.acc[k]);
+        r[2 * k + 1] = (uint32_t)__double2hiint(m.acc[k]);
+    }
+#pragma unroll
+    for (int j = 0; j < 3; ++j) r[18 + j] = (uint32_t)m.cnt[j];
+    r[21] = 0;
+    tmem_st<16>(ta + kTmemAcc, r);
+    tmem_st<2>(ta + kTmemAcc8, r + 16);
+    tmem_st<4>(ta + kTmemCnt, r + 18);
+}
+
 // Bulk launch: the run_all day loop of every cell of the tile whose spin-up is finished, one thread per cell,
 // uniform day loop (every live thread of the CTA runs days 0..n_days-1; the CTA meets at a barrier per day).
 // Thread i integrates cell p.order[i] (i < ctl->n_ready): the tile's cells regime-sorted by k_regime_*, so that
 // the cells of a warp take the same branches of the day step more often (flat / sloped, deep / shallow soil,
 // frost and snow frequency, aridity); without an order (the default: the sort was measured slower on the synthetic grid,
 // whose divergence is day-to-day weather, not regime), cell i.
+// The CTA holds its SM's TMEM (cold constants, monthly sums) from tmem_open to tmem_close, which every thread reaches.
+// TMEM instructions are warp-collective, so a lane without a cell (past the list's end, or a cell still spinning up) runs
+// the day step beside the live lanes of its warp and writes nothing; only a warp without any live lane skips it.  (Run on
+// zero constants, such lanes took the guarded divisions' slow paths every day and cost the full pass 10 %, measured.)
 template <typename FT, bool kMonthly>
 __global__ void SPLASH_BULK_BOUNDS k_run_bulk(RunParams p) {
     extern __shared__ double s_cc[];
+    __shared__ uint32_t s_tmem;
     const long long i0 = (long long)blockIdx.x * kBThreads;
     const long long n_run = p.order ? (long long)p.ctl->n_ready : (long long)p.n_cells;
-    if (i0 >= n_run) return;  // surplus CTA: all of its threads leave together
+    if (i0 >= n_run) return;  // surplus CTA: all of its threads leave together, before anything is allocated
     const long long i = i0 + threadIdx.x;
     int c = 0;
     bool live = i < n_run;
     if (live) {
         c = p.order ? p.order[i] : (int)i;
-        SPLASH_CHECK(c >= 0 && c < p.n_cells && n_run <= (long long)p.n_cells, 104);
-        live = p.w.status[c] == ST_READY_BULK;
+#ifdef SPLASH_BOUNDS_CHECK  // recorded without the early return of SPLASH_CHECK: every thread has to reach tmem_close
+        if (!(c >= 0 && c < p.n_cells && n_run <= (long long)p.n_cells)) {
+            atomicCAS(&g_bounds_err, 0ULL, 104ULL);
+            c = 0;
+            live = false;
+        }
+#endif
+        live = live && p.w.status[c] == ST_READY_BULK;
     }
+    const uint32_t ta = tmem_open(&s_tmem);
+    // A lane without a cell computes the cell of its warp's first live lane (reads only), so that it takes the same
+    // branches and adds no divergence to the warp.
+    const unsigned live_mask = __ballot_sync(0xffffffffu, live);
+    const bool warp_live = live_mask != 0;
+    const int c_run = __shfl_sync(0xffffffffu, c, live ? (int)(threadIdx.x % 32) : __ffs(live_mask) - 1);
     ShapeCC<kBThreads> cc;
-    stage_cc<kBThreads>(p, c, live, s_cc, cc);
+    stage_cc<kBThreads>(p, c_run, warp_live, s_cc, ta, cc);
     CellState st{};
-    double RES = 0.0, wrr = 1.0;
-    if (live) {
-        RES = cc(C_RES);
-        wrr = cc(C_WRR);
-        st = load_state(p.w, c);
-    }
+    if (warp_live) st = load_state(p.w, c_run);
     int n_snowfall = 0;
-    MonthAcc macc;
-    macc.clear();
+    if (kMonthly) {
+        MonthAcc m;
+        m.clear();
+        tmem_store_macc(ta, m);
+    }
+    tmem_wait_st();
     BulkForcing<FT> pipe;
-    pipe.start(p, c, live, s_cc + (size_t)staged_cc<kBThreads>() * kBThreads);
+    pipe.start(p, c_run, warp_live, s_cc + (size_t)staged_cc<kBThreads>() * kBThreads);
     for (int d = 0; d < p.n_days; ++d) {
         double f_sw, f_tc, f_pn;
-        pipe.next(p, c, d, live, f_sw, f_tc, f_pn);
+        pipe.next(p, c_run, d, warp_live, f_sw, f_tc, f_pn);
         const DayTab dt = p.dtab[d];
         if (kSync >= 1 && (d & kSyncMask) == 0) __syncthreads();
-        if (!live) continue;
+        if (!warp_live) continue;
         DayOut o;
         double rain, snowfall;
         splash_day(cc, dt, c_month_tab, f_sw, f_tc, f_pn, st, o, rain, snowfall);
         if (snowfall > 0.0) ++n_snowfall;
-#if SPLASH_BULK_RELOAD  // RES and Wmax_R - RES re-read per day: four registers less across the day step (+1.5 %, measured)
-        emit_day<kMonthly>(p, c, d, dt, cc(C_WRR), cc(C_RES), st, o, macc);
-#else
-        emit_day<kMonthly>(p, c, d, dt, wrr, RES, st, o, macc);
-#endif
+        cc_fetch(cc, CCG_OUTPUT);
+        if (kMonthly) {
+            tmem_wait_st();  // yesterday's sums
+            MonthAcc m = tmem_load_macc(ta);
+            if (live) emit_day<true>(p, c, d, dt, cc(C_WRR), cc(C_RES), st, o, m);
+            tmem_store_macc(ta, m);
+        } else if (live) {
+            MonthAcc unused;
+            emit_day<false>(p, c, d, dt, cc(C_WRR), cc(C_RES), st, o, unused);
+        }
     }
-    if (!live) return;
-    store_state(p.w, c, st);
-    if (p.diag) p.diag[SPLASH_DIAG_SNOWFALL_DAYS * p.dpitch + c] = (double)n_snowfall;
+    if (live) {
+        store_state(p.w, c, st);
+        if (p.diag) p.diag[SPLASH_DIAG_SNOWFALL_DAYS * p.dpitch + c] = (double)n_snowfall;
+    }
+    tmem_close(&s_tmem);
 }
 
 // List mode: a per-thread state machine for the few cells that outlive the lock-step rounds (the straggler pool,
@@ -1859,6 +2034,10 @@ inline unsigned bgrid_for(int64_t n) { return (unsigned)((n + kBThreads - 1) / k
 constexpr size_t kSmemBulkF32 = kSmemBulkCC + sizeof(float) * 2 * 3 * kBThreads;  // f32 forcing: + the cp.async ring
 template <typename FT> constexpr size_t bulk_smem() { return sizeof(FT) == 4 ? kSmemBulkF32 : kSmemBulkCC; }
 static_assert(kSmemBulkF32 <= 227 * 1024, "bulk launch: shared memory per CTA");
+// More than half of the SM's 228 KB: two bulk CTAs, each allocating all of the SM's TMEM, can never share an SM, so
+// tcgen05.alloc never waits for another CTA's columns (no other kernel allocates TMEM).
+static_assert(kSmemBulkCC > 228 * 1024 / 2, "bulk launch: one CTA per SM");
+static_assert((kBThreads / 32 + 3) / 4 * kTmemSlice <= kTmemCols && kBThreads % 32 == 0, "bulk launch: TMEM columns per warp");
 constexpr size_t kSmemList = sizeof(double) * (NCC_DAY + 5) * kListThreads;  // list mode: + cycle snapshot
 
 template <typename FT>

@@ -116,6 +116,13 @@ enum CellConst : int {
 #endif
 };
 
+// Sections of day_forcing that read constants an accessor may keep outside its directly addressable storage: the bulk
+// launch holds them in tensor memory and moves each group into registers at the top of its section (splash_cuda.cu,
+// TmemCC).  day_forcing calls cc_fetch where every lane of a warp reaches it; accessors without such storage ignore it.
+enum CCGroup : int { CCG_SNOW, CCG_GEOMETRY, CCG_PRESSURE, CCG_OUTPUT };
+template <class CC>
+__device__ __forceinline__ void cc_fetch(const CC&, CCGroup) {}
+
 struct DayTab {      // per-day values that do not depend on the cell (host-built, SOLAR.cpp:98-124)
     double dr;       // distance factor
     double sd;       // sin(delta*pir)
@@ -516,6 +523,7 @@ template <class M = MathShared, class CC>
 __device__ __forceinline__ void day_forcing(const CC& cc, const DayTab& dt, const MonthTab& mt, double sw_in, double tc,
                                             double pn, DayPre& q) {
     // ---- snow partition, R/splash.point.R:120-128 with frain_func :547-555 ------------------------
+    cc_fetch(cc, CCG_SNOW);  // C_ELEV_K, C_LAT_K, C_TT
     const int snowy = snow_class(cc, tc);
     double f_rain;
     if (snowy < 0) {
@@ -541,6 +549,7 @@ __device__ __forceinline__ void day_forcing(const CC& cc, const DayTab& dt, cons
     q.tc = tc;
 
     // ---- SOLAR::calculate_daily_fluxes, SOLAR.cpp:129-203 ------------------------------------------
+    cc_fetch(cc, CCG_GEOMETRY);  // the six trig constants, C_TAU_O, C_TAU_A, C_INV_TAU_B
     const double a = dt.sd * cc(C_COS_LAT) * cc(C_SIN_S) * cc(C_COS_A) - dt.sd * cc(C_SIN_LAT) * cc(C_COS_S);
     const double b = dt.cd * cc(C_COS_LAT) * cc(C_COS_S) + dt.cd * cc(C_SIN_LAT) * cc(C_SIN_S) * cc(C_COS_A);
     const double c = dt.cd * cc(C_SIN_S) * cc(C_SIN_A);
@@ -613,6 +622,7 @@ __device__ __forceinline__ void day_forcing(const CC& cc, const DayTab& dt, cons
     q.rw_dark = ((sw_in == 0.0) || (hs == 0.0)) ? 1.0 : 0.0;
 
     // ---- EVAP::calculate_daily_fluxes, EVAP.cpp:100-145 --------------------------------------------
+    cc_fetch(cc, CCG_PRESSURE);  // C_PATM, C_PBAR, C_PBARF, C_VISC0, C_INTPERM
     const double patm = cc(C_PATM);
     double s = M::exp(SPLASH_FDIV(tc * kD.ss_a, tc + kD.ss_b));  // sat_slope, :299-301
     s = SPLASH_FDIV(s, (tc + kD.ss_b) * (tc + kD.ss_b));
