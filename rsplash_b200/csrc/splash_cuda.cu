@@ -11,9 +11,8 @@
 //                     the list sizes stay on the device, the host never waits for them
 //   k_run_bulk        the run_all day loop of every cell whose spin-up is finished: 768 threads per SM, state in
 //                     registers, the state half's constants in shared memory and the forcing half's in tensor
-//                     memory (TmemCC), optionally in regime-sorted order (k_regime_*), next day's
-//                     forcing staged by cp.async, outputs written with streaming stores (daily) or reduced per
-//                     month in tensor memory (monthly)
+//                     memory (TmemCC), next day's forcing staged by cp.async, outputs written with streaming
+//                     stores (daily) or reduced per month in tensor memory (monthly)
 //   k_run_list        per-thread state machine (rest of the spin-up, then the day loop) for the few cells
 //                     that outlive the lock-step passes; lanes fetch cells from a device-side queue
 //   k_pool_*          move those stragglers (constants, state, forcing columns) into a context-wide
@@ -54,61 +53,20 @@ using namespace splash;
 namespace {
 
 constexpr int kThreads = 128;  // threads per CTA of the list-mode (non-uniform) day-loop kernels
-#ifndef SPLASH_MIN_BLOCKS
-#define SPLASH_MIN_BLOCKS 4
-#endif
-constexpr int kMinBlocks = SPLASH_MIN_BLOCKS;  // resident CTAs per SM the register allocation aims for
-// Uniform kernels (every thread of the CTA runs the same days): one large CTA per SM whose warps are
-// kept together by a CTA barrier per day (SPLASH_SYNC=1; 0 = none), so that they walk through the ~60 KB
-// loop body together and share instruction-cache lines instead of each streaming the body from L2 on
-// its own (the body is larger than the 32 KB L1.5 instruction cache; profiles/README.md).
-#ifndef SPLASH_SYNC
-#define SPLASH_SYNC 1
-#endif
-#ifndef SPLASH_UTHREADS
-#define SPLASH_UTHREADS 512
-#endif
-#ifndef SPLASH_UBLOCKS
-#define SPLASH_UBLOCKS 1
-#endif
+constexpr int kMinBlocks = 4;  // resident CTAs per SM the register allocation aims for
 constexpr int kListThreads = 32;  // list mode: one warp per CTA, so that the few long-running warps spread over all SMs
-#ifndef SPLASH_SYNC_EVERY
-#define SPLASH_SYNC_EVERY 1  // barrier every n-th day (power of two)
-#endif
-constexpr int kSyncMask = SPLASH_SYNC_EVERY - 1;
-constexpr int kSync = SPLASH_SYNC;
-constexpr int kUThreads = SPLASH_UTHREADS;
-constexpr int kUBlocks = SPLASH_UBLOCKS;
-// Register budget of the uniform kernels: they are compiled for a CTA `kURegSlack` threads larger than
-// the one launched, so that a full CTA leaves room on its SM for one-warp CTAs of the straggler pool
-// (list mode, 128 registers/thread).  Without the slack a 512-thread CTA owns the whole register file
-// and the long-running pool warps and the uniform kernels would exclude each other from an SM.
-#ifndef SPLASH_UREG_SLACK
-#define SPLASH_UREG_SLACK 64
-#endif
-constexpr int kUBound = kUThreads + SPLASH_UREG_SLACK;
-// SPLASH_UREGS: the register cap of the uniform kernels.  A full 512-thread CTA at 104 registers leaves 12 288 registers
+// Uniform kernels (every thread of the CTA runs the same days): one large CTA per SM whose warps are
+// kept together by a CTA barrier per day, so that they walk through the ~60 KB loop body together and
+// share instruction-cache lines instead of each streaming the body from L2 on its own (the body is larger
+// than the 32 KB L1.5 instruction cache; profiles/README.md).  The literal-order day step (SPLASH_LEVEL=0)
+// keeps 57 constants per cell in shared memory: 448 cells fit a CTA, 512 do not.
+constexpr int kUThreads = SPLASH_L1_RECIP ? 512 : 448;
+// The register cap of the uniform kernels.  A full 512-thread CTA at 104 registers leaves 12 288 registers
 // of its SM free: three one-warp CTAs of the straggler pool (128 registers per thread).  Measured on the resident
 // benchmark (profiles/README.md): 96 registers (what a launch bound of 576 threads gives) 3.09 s per pass, 104: 2.92 s,
 // 112 / 120 / 128: faster bulk kernel alone (up to +15 %) but 3.1 - 3.9 s per pass, because pool warps and such CTAs then
-// exclude each other from an SM and the straggler chain ends after the bulk launches.  SPLASH_UREGS=0: launch bound.
-#ifndef SPLASH_UREGS
-#define SPLASH_UREGS (SPLASH_UTHREADS > 512 ? 80 : 104)
-#endif
-// the bulk launch (k_run_bulk) has its own shape, see kBThreads below (the literal-order day step, SPLASH_LEVEL=0, reads
-// five more constants per cell: its 39 hot ones do not fit 768 threads, so it keeps the shape of the other kernels)
-#ifndef SPLASH_BULK_THREADS
-#define SPLASH_BULK_THREADS (SPLASH_L1_RECIP ? 768 : SPLASH_UTHREADS)
-#endif
-#ifndef SPLASH_BULK_REGS
-#define SPLASH_BULK_REGS (SPLASH_BULK_THREADS > 512 ? 80 : 104)
-#endif
-#define SPLASH_BULK_BOUNDS __maxnreg__(SPLASH_BULK_REGS)
-#if SPLASH_UREGS > 0
-#define SPLASH_UNIFORM_BOUNDS __maxnreg__(SPLASH_UREGS)
-#else
-#define SPLASH_UNIFORM_BOUNDS __launch_bounds__(kUBound, kUBlocks)
-#endif
+// exclude each other from an SM and the straggler chain ends after the bulk launches.
+constexpr int kURegs = 104;
 constexpr int kSpinYear = 365; // R/splash.point.R:141-152: the spin-up year is always 365 days
 
 __constant__ MonthTab c_month_tab;
@@ -147,7 +105,10 @@ struct StridedCC {  // column of a [NCC][stride] matrix (shared or global memory
 // stage use in the thread's tensor-memory columns (TmemCC), from where each section of the day step loads its group.
 // The bulk launch runs 768 threads x 80 registers = six warps per scheduler (+8 % on the kernel alone, measured; the
 // spin-up kernels keep 512 threads: their late rounds are short lists, where larger CTAs were measured slower).
-constexpr int kBThreads = SPLASH_BULK_THREADS;
+// The literal-order day step reads five more constants per cell: its 39 hot ones do not fit 768 threads, so its bulk
+// launch keeps the shape of the uniform kernels.
+constexpr int kBThreads = SPLASH_L1_RECIP ? 768 : kUThreads;
+constexpr int kBRegs = kBThreads > 512 ? 80 : 104;
 template <int NT> __host__ __device__ constexpr bool hybrid_cc() { return NT > 512; }
 
 // Constants that only day_forcing (and the output stage) read, with their slots, the order of their tensor-memory columns
@@ -357,19 +318,18 @@ __global__ void __launch_bounds__(128) k_cell_setup(SetupParams p) {
 template <typename FT>
 __global__ void __launch_bounds__(256) k_snow_threshold(const FT* __restrict__ tc, int64_t fpitch, int n_days,
                                                         int n_cells, double* cc, int64_t cpitch, double* diag,
-                                                        int64_t dpitch, int* frost) {
+                                                        int64_t dpitch) {
     const int c = blockIdx.x * blockDim.x + threadIdx.x;
     if (c >= n_cells) return;
     StridedCC ccg{cc + c, cpitch};
     // Tt <- max(tc[p_snow >= 0.5]); an NA probability makes the result NA, an empty set gives -Inf
     double Tt = -INFINITY;
     bool any_na = false;
-    int n_snow = 0, n_frost = 0;
+    int n_snow = 0;
     const FT* col = tc + c;
 #pragma unroll 4
     for (int d = 0; d < n_days; ++d) {
         const double t = ld_stream(col + (int64_t)d * fpitch);
-        n_frost += (t < 0.0) ? 1 : 0;
         const int snowy = snow_class(ccg, t);
         if (snowy < 0) {
             any_na = true;
@@ -380,7 +340,6 @@ __global__ void __launch_bounds__(256) k_snow_threshold(const FT* __restrict__ t
     }
     if (any_na) Tt = nan("");
     ccg(C_TT) = Tt;
-    if (frost) frost[c] = n_frost;
     if (diag) {
         diag[SPLASH_DIAG_TT * dpitch + c] = Tt;
         diag[SPLASH_DIAG_SNOW_DAYS * dpitch + c] = (double)n_snow;
@@ -400,7 +359,6 @@ __global__ void __launch_bounds__(256) k_snow_threshold(const FT* __restrict__ t
 // ---------------------------------------------------------------------------------------------
 enum : int { ST_ACTIVE = 0, ST_READY_BULK = 1, ST_EXPORTED = 3 };
 constexpr int kMaxRounds = 32;  // upper bound of lock-step year passes per tile
-constexpr int kRegimeKeys = 128; // buckets of the regime sort (k_regime_*)
 
 // Device-resident control block of one tile.  Everything the kernels of a tile need to know about
 // the sizes of its lists lives here, so the host enqueues the whole tile without waiting.
@@ -416,8 +374,6 @@ struct TileCtl {
     unsigned long long decl_n, decl_head;    // cells of the last stage that keep declining the branch-light day step (guarded route)
     unsigned long long tail_head, tail_end;  // leftovers that did not fit the pool: finished in the tile
     unsigned long long max_chain;            // most year passes executed by one thread of a list-mode launch
-    unsigned long long n_ready;              // cells in the regime-sorted order of the bulk launch
-    unsigned long long regime[kRegimeKeys];  // regime sort: bucket counts, then bucket cursors
 };
 
 struct Work {
@@ -427,8 +383,6 @@ struct Work {
     int* passes;
     int* snap_pass;
     int* status;
-    int* frost;          // days with tc < 0 (k_snow_threshold): a key of the regime sort (null in the pool's view)
-    unsigned char* key;  // regime-sort bucket of the cell
     int64_t pitch;
 };
 
@@ -447,8 +401,6 @@ struct RunParams {
     int n_cells;               // cells of the tile
     Work w;
     int* lists[2];             // ping-pong spin lists of the tile: list r lives in lists[r & 1] (list 0 = identity)
-    const int* order;          // k_run_bulk: regime-sorted cell order (ctl->n_ready entries); null = identity
-    int* order_w;              // ... as written by k_regime_scatter
     int round;                 // k_spin_check / k_spin_rest: lock-step round r
     TileCtl* ctl;              // the tile's control block
     // k_run_list: lanes fetch i from *q_head while i < *q_end; cell = q_list ? q_list[i] : i
@@ -702,7 +654,7 @@ __device__ __forceinline__ void apply_lateral(const RunParams& p, int c, double*
 
 // ---- K2a: aridity pass + pass 0 of the second spin_up, all cells, 730 uniform days ---------------
 template <typename FT>
-__global__ void SPLASH_UNIFORM_BOUNDS k_spin_first(RunParams p) {
+__global__ void __maxnreg__(kURegs) k_spin_first(RunParams p) {
     extern __shared__ double s_cc[];
     const int c = blockIdx.x * kUThreads + threadIdx.x;
     const bool live = c < p.n_cells;  // threads past the tile's end idle through the loop: every thread reaches every barrier
@@ -725,7 +677,7 @@ __global__ void SPLASH_UNIFORM_BOUNDS k_spin_first(RunParams p) {
         const DayTab dt = p.dtab_spin[d];
         DayOut o;
         double rain, snowfall;
-        if (kSync >= 1 && (it & kSyncMask) == 0) __syncthreads();
+        __syncthreads();
         if (!live) continue;
         splash_day(cc, dt, c_month_tab, f_sw, f_tc, f_pn, st, o, rain, snowfall);
         if (it < kSpinYear) {
@@ -796,7 +748,7 @@ __global__ void __launch_bounds__(kThreads, kMinBlocks) k_spin_check(RunParams p
 
 // ---- K2c: days 2..365 of a year pass for the (compacted) cells that continue ----------------------
 template <typename FT>
-__global__ void SPLASH_UNIFORM_BOUNDS k_spin_rest(RunParams p) {
+__global__ void __maxnreg__(kURegs) k_spin_rest(RunParams p) {
     extern __shared__ double s_cc[];
     const int r = p.round;
     const unsigned long long i = (unsigned long long)blockIdx.x * kUThreads + threadIdx.x;
@@ -818,7 +770,7 @@ __global__ void SPLASH_UNIFORM_BOUNDS k_spin_rest(RunParams p) {
         const DayTab dt = p.dtab_spin[d];
         DayOut o;
         double rain, snowfall;
-        if (kSync >= 1 && (d & kSyncMask) == 0) __syncthreads();
+        __syncthreads();
         if (!live) continue;
         splash_day(cc, dt, c_month_tab, f_sw, f_tc, f_pn, st, o, rain, snowfall);
     }
@@ -904,37 +856,22 @@ __device__ __forceinline__ void tmem_store_macc(uint32_t ta, const MonthAcc& m) 
     tmem_st<4>(ta + kTmemCnt, r + 18);
 }
 
-// Bulk launch: the run_all day loop of every cell of the tile whose spin-up is finished, one thread per cell,
-// uniform day loop (every live thread of the CTA runs days 0..n_days-1; the CTA meets at a barrier per day).
-// Thread i integrates cell p.order[i] (i < ctl->n_ready): the tile's cells regime-sorted by k_regime_*, so that
-// the cells of a warp take the same branches of the day step more often (flat / sloped, deep / shallow soil,
-// frost and snow frequency, aridity); without an order (the default: the sort was measured slower on the synthetic grid,
-// whose divergence is day-to-day weather, not regime), cell i.
+// Bulk launch: the run_all day loop of every cell of the tile whose spin-up is finished, one thread per cell (thread i
+// integrates cell i), uniform day loop (every live thread of the CTA runs days 0..n_days-1; the CTA meets at a barrier
+// per day).
 // The CTA holds its SM's TMEM (cold constants, monthly sums) from tmem_open to tmem_close, which every thread reaches.
-// TMEM instructions are warp-collective, so a lane without a cell (past the list's end, or a cell still spinning up) runs
+// TMEM instructions are warp-collective, so a lane without a cell (past the tile's end, or a cell still spinning up) runs
 // the day step beside the live lanes of its warp and writes nothing; only a warp without any live lane skips it.  (Run on
 // zero constants, such lanes took the guarded divisions' slow paths every day and cost the full pass 10 %, measured.)
 template <typename FT, bool kMonthly>
-__global__ void SPLASH_BULK_BOUNDS k_run_bulk(RunParams p) {
+__global__ void __maxnreg__(kBRegs) k_run_bulk(RunParams p) {
     extern __shared__ double s_cc[];
     __shared__ uint32_t s_tmem;
     const long long i0 = (long long)blockIdx.x * kBThreads;
-    const long long n_run = p.order ? (long long)p.ctl->n_ready : (long long)p.n_cells;
-    if (i0 >= n_run) return;  // surplus CTA: all of its threads leave together, before anything is allocated
+    if (i0 >= p.n_cells) return;  // surplus CTA: all of its threads leave together, before anything is allocated
     const long long i = i0 + threadIdx.x;
-    int c = 0;
-    bool live = i < n_run;
-    if (live) {
-        c = p.order ? p.order[i] : (int)i;
-#ifdef SPLASH_BOUNDS_CHECK  // recorded without the early return of SPLASH_CHECK: every thread has to reach tmem_close
-        if (!(c >= 0 && c < p.n_cells && n_run <= (long long)p.n_cells)) {
-            atomicCAS(&g_bounds_err, 0ULL, 104ULL);
-            c = 0;
-            live = false;
-        }
-#endif
-        live = live && p.w.status[c] == ST_READY_BULK;
-    }
+    const int c = i < p.n_cells ? (int)i : 0;
+    const bool live = i < p.n_cells && p.w.status[c] == ST_READY_BULK;
     const uint32_t ta = tmem_open(&s_tmem);
     // A lane without a cell computes the cell of its warp's first live lane (reads only), so that it takes the same
     // branches and adds no divergence to the warp.
@@ -958,7 +895,7 @@ __global__ void SPLASH_BULK_BOUNDS k_run_bulk(RunParams p) {
         double f_sw, f_tc, f_pn;
         pipe.next(p, c_run, d, warp_live, f_sw, f_tc, f_pn);
         const DayTab dt = p.dtab[d];
-        if (kSync >= 1 && (d & kSyncMask) == 0) __syncthreads();
+        __syncthreads();
         if (!warp_live) continue;
         DayOut o;
         double rain, snowfall;
@@ -1085,57 +1022,6 @@ __global__ void __launch_bounds__(kListThreads, 16) k_run_list(RunParams p) {
     if (max_chain) atomicMax(&p.ctl->max_chain, (unsigned long long)max_chain);
 }
 
-// ---- regime sort: a counting sort of the tile's finished cells by a key that predicts which branches of the
-//      day step a cell takes (k_run_bulk runs the cells in this order; results do not depend on it) -------------
-__device__ __forceinline__ int regime_key(const RunParams& p, int c) {
-    const double tan_s = p.cc[(int64_t)C_TAN_S * p.cpitch + c];
-    const double depth = p.cc[(int64_t)C_DEPTH * p.cpitch + c];
-    const double ai = p.cc[(int64_t)C_CELLOUT * p.cpitch + c];  // the aridity index sits in the cellout slot (SURVEY B-3)
-    const double sat = p.cc[(int64_t)C_SAT * p.cpitch + c];
-    if (isnan(sat) || isnan(ai) || isnan(tan_s)) return kRegimeKeys - 1;  // NA cells together
-    const int flat = (tan_s == 0.0) ? 1 : 0;
-    const int deep = (depth >= 2.0) ? 1 : 0;
-    const int nd = p.n_days > 0 ? p.n_days : 1;
-    const int frost = p.w.frost[c];  // days with tc < 0 (viscosity is a cell constant there), k_snow_threshold
-    const int fq = (frost == 0) ? 0 : ((8 * (long long)frost) / nd >= 7 ? 3 : ((2 * (long long)frost >= nd) ? 2 : 1));
-    const int wq = (ai < 0.6) ? 0 : (ai < 1.2) ? 1 : (ai < 2.5) ? 2 : 3;  // humid ... arid
-    return ((flat * 2 + deep) * 4 + fq) * 4 + wq;  // 0..63
-}
-
-__global__ void __launch_bounds__(256) k_regime_count(RunParams p) {
-    __shared__ unsigned int h[kRegimeKeys];
-    for (int k = threadIdx.x; k < kRegimeKeys; k += blockDim.x) h[k] = 0;
-    __syncthreads();
-    const int c = blockIdx.x * blockDim.x + threadIdx.x;
-    if (c < p.n_cells && p.w.status[c] == ST_READY_BULK) {
-        const int key = regime_key(p, c);
-        p.w.key[c] = (unsigned char)key;
-        atomicAdd(&h[key], 1u);
-    }
-    __syncthreads();
-    for (int k = threadIdx.x; k < kRegimeKeys; k += blockDim.x)
-        if (h[k]) atomicAdd(&p.ctl->regime[k], (unsigned long long)h[k]);
-}
-
-__global__ void k_regime_scan(TileCtl* ctl) {  // one thread: bucket counts -> bucket cursors
-    unsigned long long run = 0;
-    for (int k = 0; k < kRegimeKeys; ++k) {
-        const unsigned long long n = ctl->regime[k];
-        ctl->regime[k] = run;
-        run += n;
-    }
-    ctl->n_ready = run;
-}
-
-__global__ void __launch_bounds__(256) k_regime_scatter(RunParams p) {
-    const int c = blockIdx.x * blockDim.x + threadIdx.x;
-    if (c < p.n_cells && p.w.status[c] == ST_READY_BULK) {
-        const unsigned long long k = atomicAdd(&p.ctl->regime[p.w.key[c]], 1ULL);
-        SPLASH_CHECK(p.w.key[c] < kRegimeKeys && k < (unsigned long long)p.n_cells, 106);
-        p.order_w[k] = c;
-    }
-}
-
 // ---------------------------------------------------------------------------------------------
 // Straggler pool.  The cells still spinning after a tile's lock-step rounds (a fraction of a
 // percent, but each may need up to 1000 year passes) are copied out of the tile -- constants, work
@@ -1237,7 +1123,9 @@ __global__ void __launch_bounds__(128) k_pool_table(RunParams p, Pool pool) {
         spin_forcing<FT>(p, j, d, f_sw, f_tc, f_pn);
         DayPre pre;
         day_forcing(cc, p.dtab_spin[d], c_month_tab, f_sw, f_tc, f_pn, pre);
+#if SPLASH_L1_RECIP  // (the literal-order build has no branch-light day step to read these terms)
         day_forcing_recession(cc, pre);
+#endif
         const double* v = reinterpret_cast<const double*>(&pre);
         double* dst = pool.table + ((long long)j * kSpinYear + d) * kDayPrePad;
 #pragma unroll
@@ -1246,15 +1134,6 @@ __global__ void __launch_bounds__(128) k_pool_table(RunParams p, Pool pool) {
 }
 
 constexpr int kFastDeclineLimit = 36;  // days of the probe pass (10 %) the branch-light route may decline before the cell goes to the guarded list
-// SPLASH_CHAIN_FAST: the chain's state half through the branch-light route (day_state_fast, splash_model.cuh)
-#ifndef SPLASH_CHAIN_FAST
-#define SPLASH_CHAIN_FAST 1
-#endif
-#ifdef SPLASH_CHAIN_SHARED_MATH
-using ChainMath = MathShared;
-#else
-using ChainMath = MathInline;
-#endif
 
 // The rest of the second spin_up call (SPLASH.cpp:1697-1743) for the pool's cells: a per-thread loop over
 // year passes with the reference's convergence test and exact cycle detection, the forcing half of every
@@ -1269,7 +1148,7 @@ using ChainMath = MathInline;
 // uniform kernels fits beside it: its warps (at most four per SM) own their SM and run the chain at
 // its uncontended latency, roughly half the time per day step of a warp squeezed in beside 16 others.
 //
-// kBoth (the last stage when SPLASH_CHAIN_FAST): the state half through day_state_fast (splash_model.cuh), which
+// kBoth (the last stage unless SPLASH_CHAIN_FAST=0): the state half through day_state_fast (splash_model.cuh), which
 // shortens a lone warp's dependent chain by ~1.7x -- for the cells whose days stay inside its fast ranges.  A cell
 // that keeps declining it (a column at its residual moisture, a zero air-entry pressure ...) would pay for both
 // routes every day, and so would its warp.  So the last stage is two launches: a PROBE (stage 3) runs one year pass
@@ -1359,9 +1238,9 @@ __global__ void __launch_bounds__(kListThreads, kBoth ? 8 : 16) k_pool_spin(RunP
             if (d == 0) saved = st;  // E_k: state of day 365 before the check day
             DayOut o;
             if constexpr (kBoth) {
-                declined += day_state_auto<ChainMath>(cc, pre, st, o, fast) ? 0 : 1;
+                declined += day_state_auto<MathInline>(cc, pre, st, o, fast) ? 0 : 1;
             } else {
-                day_state<ChainMath>(cc, pre, st, o);
+                day_state<MathInline>(cc, pre, st, o);
             }
             ++spin_days;
             if (d == 0) {
@@ -1490,7 +1369,7 @@ __global__ void __launch_bounds__(256) k_unswc(UnswcParams p) {
         } else {
             theta_i = (theta_o <= theta_r) ? theta_r + 0.0001 : theta_o;
         }
-#if SPLASH_LEVEL >= 1 && !defined(SPLASH_LIBDEVICE_MATH)
+#if SPLASH_LEVEL >= 1
         // x^y as exp(y*log(x)) with the library's own exp/log (level-1 arithmetic, DESIGN.md)
         const double x = ((theta_i - theta_r) / (theta_s - theta_r));
         const double psi_m = bub / fm::pow_core(x, ilam);  // :109
@@ -1503,7 +1382,7 @@ __global__ void __launch_bounds__(256) k_unswc(UnswcParams p) {
         const bool na2 = isnan(wtd2) || isnan(ud);
         const bool shallow = !na2 && (wtd2 <= ud);
         const double z_uns = na2 ? nan("") : (shallow ? wtd2 * 1000 : ud * 1000);
-#if SPLASH_LEVEL >= 1 && !defined(SPLASH_LIBDEVICE_MATH)
+#if SPLASH_LEVEL >= 1
         // both powers through the same function: at z_uns == 0 the two terms must cancel exactly, as in R
         const double pz = fm::pow_core(bub / (psi_m + z_uns), lambda);
         const double p0 = fm::pow_core(bub / (psi_m + 0), lambda);
@@ -1916,10 +1795,7 @@ constexpr int kSlots = 3;         // forcing / output buffer sets in flight when
 constexpr int kRunStreams = 8;    // compute streams the tiles are dealt to
 constexpr int kPoolStreams = 16;  // streams of the straggler-pool launches: a tile's pool work must not queue behind
                                   // another tile's seconds-long chain, so calls are cut into at most 16 tiles when possible
-#ifndef SPLASH_ROUNDS
-#define SPLASH_ROUNDS 20
-#endif
-constexpr int kRounds = SPLASH_ROUNDS;  // lock-step year passes per tile before the leftovers go to the pool
+constexpr int kRounds = 20;  // lock-step year passes per tile before the leftovers go to the pool
 // Pass budgets of the pool's first two spin-up stages and the shape of the third, which runs to the reference's pass
 // limit on SMs of its own.  Two presets, chosen per call by its size (profiles/README.md R2.2):
 //   large calls (the straggler chain hides behind seconds of bulk work): 8 / 128 passes, 16 cells per last-stage warp on 48
@@ -1933,12 +1809,9 @@ constexpr double kPoolSmallCallCellDays = 5e9;  // n_cells * n_days below which 
 static_assert(kRounds <= kMaxRounds, "kRounds");
 // cells per tile aimed for: two full waves of the 512-thread uniform kernels (the bulk launches of several tiles run side
 // by side on their streams, so a 768-thread bulk CTA shape needs no whole number of waves per tile)
-#ifndef SPLASH_TILE_TARGET
-#define SPLASH_TILE_TARGET (148LL * 512 * 2)
-#endif
-constexpr int64_t kTileTarget = SPLASH_TILE_TARGET;
+constexpr int64_t kTileTarget = 148LL * 512 * 2;
 
-constexpr int kWorkInts = 8;  // int arrays of a work set: passes, snap_pass, status, 2 spin lists, frost days, bulk order, sort keys
+constexpr int kWorkInts = 5;  // int arrays of a work set: passes, snap_pass, status, 2 spin lists
 struct WorkSet {  // per-tile work arrays (per slot when the inputs stream from the host)
     DevBuf cc, work_d, work_i, diag;
 };
@@ -1961,19 +1834,14 @@ struct splash_ctx {
     std::vector<WorkSet> work;
     DevBuf dtab, dtab_spin, ctl, pool_mem, ahead_mem;
     // tuning knobs (environment overrides for experiments, read once at creation)
-    int n_run_streams = kRunStreams;      // SPLASH_RUN_STREAMS
     int pool_stage1 = kPoolStage1Passes;  // SPLASH_POOL_STAGE1 (0 = single stage)
     int pool_stage2 = kPoolStage2Passes;  // SPLASH_POOL_STAGE2
-    int pool_excl_smem = 0;               // dynamic shared memory of a last-stage CTA (SPLASH_POOL_EXCL=0: no exclusivity)
+    int pool_excl_smem = 0;               // dynamic shared memory of a last-stage CTA (a quarter of the SM's)
     int pool_last_lanes = kPoolLastLanes, pool_last_ctas = kPoolLastCtas;  // SPLASH_POOL_LANES, SPLASH_POOL_CTAS
-    int chain_fast = SPLASH_CHAIN_FAST;  // SPLASH_CHAIN_FAST=0/1: the pool's last stage on the branch-light day step (k_pool_spin)
+    bool chain_fast = true;               // SPLASH_CHAIN_FAST=0/1: the pool's last stage on the branch-light day step (k_pool_spin)
     bool pool_auto = true;                // none of the four was set in the environment: preset by call size
-    int two_pass = 1;                     // SPLASH_TWO_PASS
     int n_rounds = kRounds;               // SPLASH_ROUNDS_RT (<= kRounds)
     int64_t pool_cap = 0;                 // SPLASH_POOL_CAP: force the pool capacity (tests of the overflow path)
-    int spin_ahead = 1;                   // SPLASH_SPIN_AHEAD=0: host-fed calls upload tile by tile (no spin-up data first)
-    int regime_sort = 0;                  // SPLASH_REGIME_SORT=1: the bulk launch takes the cells in regime-sorted order (measured
-                                          // slower on the synthetic grid, whose divergence is day-to-day weather: profiles/README.md)
     double mem_share = 1.0;               // share of the device's memory this context may plan with (lanes of a cluster)
     // a context over several GPUs (splash_ctx_create_multi): the work goes to the cluster's lanes
     splash_cluster* multi = nullptr;
@@ -2123,10 +1991,8 @@ int splash_ctx_create(int device, splash_ctx** out_ctx) {
 static int ctx_create_impl(int device, splash_ctx* ctx, const cudaDeviceProp& prop) {
     ctx->device = device;
     ctx->sm_count = prop.multiProcessorCount;
-    if (const char* v = getenv("SPLASH_RUN_STREAMS")) ctx->n_run_streams = std::max(1, std::min(kRunStreams, atoi(v)));
     ctx->pool_auto = !getenv("SPLASH_POOL_STAGE1") && !getenv("SPLASH_POOL_STAGE2") && !getenv("SPLASH_POOL_LANES") && !getenv("SPLASH_POOL_CTAS");
     if (const char* v = getenv("SPLASH_POOL_STAGE1")) ctx->pool_stage1 = std::max(0, atoi(v));
-    if (const char* v = getenv("SPLASH_TWO_PASS")) ctx->two_pass = atoi(v) != 0;
     if (const char* v = getenv("SPLASH_POOL_STAGE2")) ctx->pool_stage2 = std::max(1, atoi(v));
     if (const char* v = getenv("SPLASH_POOL_LANES")) ctx->pool_last_lanes = std::max(1, std::min(32, atoi(v)));
     if (const char* v = getenv("SPLASH_CHAIN_FAST")) ctx->chain_fast = atoi(v) != 0;
@@ -2134,27 +2000,19 @@ static int ctx_create_impl(int device, splash_ctx* ctx, const cudaDeviceProp& pr
     {
         // a quarter of the SM's shared memory per last-stage CTA: four of them fill an SM, and none fits
         // beside a uniform CTA (kSmemUniform)
-        const char* v = getenv("SPLASH_POOL_EXCL");
-        const bool excl = !v || atoi(v) != 0;
         const int quarter = ((int)prop.sharedMemPerMultiprocessor - 4 * 1024) / 4 / 1024 * 1024;
-        ctx->pool_excl_smem = excl ? std::max<int>((int)kSmemList, std::min<int>(quarter, (int)prop.sharedMemPerBlockOptin)) : (int)kSmemList;
+        ctx->pool_excl_smem = std::max<int>((int)kSmemList, std::min<int>(quarter, (int)prop.sharedMemPerBlockOptin));
     }
     if (const char* v = getenv("SPLASH_ROUNDS_RT")) ctx->n_rounds = std::max(0, std::min(kRounds, atoi(v)));
     if (const char* v = getenv("SPLASH_POOL_CAP")) ctx->pool_cap = std::max<int64_t>(32, atoll(v));
-    if (const char* v = getenv("SPLASH_SPIN_AHEAD")) ctx->spin_ahead = atoi(v) != 0;
-    if (const char* v = getenv("SPLASH_REGIME_SORT")) ctx->regime_sort = atoi(v) != 0;
     CU(cudaSetDevice(device));
     int prio_lo = 0, prio_hi = 0;
     CU(cudaDeviceGetStreamPriorityRange(&prio_lo, &prio_hi));
     CU(cudaStreamCreateWithFlags(&ctx->s_h2d, cudaStreamNonBlocking));
     CU(cudaStreamCreateWithFlags(&ctx->s_d2h, cudaStreamNonBlocking));
-    // Stragglers first (the chain of the slowest cell is the critical path of a call); the tiles abreast.
-    // SPLASH_TILE_PRIO=1 ranks tile t's stream above tile t+1's (earlier chain starts for the first tiles): measured
-    // WORSE on the resident benchmark (4.0 - 4.5 s per pass against 2.9 s: the later tiles' spin-ups starve and their
-    // chains end after everything else), kept as a knob only.
-    const bool tile_prio = getenv("SPLASH_TILE_PRIO") && atoi(getenv("SPLASH_TILE_PRIO")) != 0;
-    for (int i = 0; i < kRunStreams; ++i)
-        CU(cudaStreamCreateWithPriority(&ctx->s_run[i], cudaStreamNonBlocking, tile_prio ? std::min(prio_lo, prio_hi + 1 + i) : prio_lo));
+    // Stragglers first (the chain of the slowest cell is the critical path of a call); the tiles abreast: ranking
+    // tile t above tile t+1 starves the later tiles' spin-ups and ends their chains last (measured slower).
+    for (auto& s : ctx->s_run) CU(cudaStreamCreateWithPriority(&s, cudaStreamNonBlocking, prio_lo));
     for (auto& s : ctx->s_pool) CU(cudaStreamCreateWithPriority(&s, cudaStreamNonBlocking, prio_hi));
     k_init_tables<<<(kSnowAgeTab + 255) / 256, 256>>>();
     CU(cudaGetLastError());
@@ -2893,7 +2751,7 @@ struct GridJob {
     cudaEvent_t ev_begin = nullptr, ev_end = nullptr;
 
     TileCtl* ctl(int64_t t) const { return (TileCtl*)ctx->ctl.p + t; }
-    cudaStream_t run_stream(int64_t t) const { return ctx->s_run[t % ctx->n_run_streams]; }
+    cudaStream_t run_stream(int64_t t) const { return ctx->s_run[t % kRunStreams]; }
     int work_of(int64_t t) const { return (in_dev || ahead) ? (int)t : (int)(t % kSlots); }
     int64_t cells_of(int64_t t) const { return std::min<int64_t>(tile, nc - t * tile); }
 
@@ -2949,8 +2807,6 @@ struct GridJob {
             pool.w.passes = wi;
             pool.w.snap_pass = wi + cap;
             pool.w.status = wi + 2 * cap;
-            pool.w.frost = nullptr;
-            pool.w.key = nullptr;
             pool.w.pitch = cap;
             int li = 0;
             for (int k = 0; k < 9; ++k)
@@ -2975,7 +2831,7 @@ struct GridJob {
             const double left = budget - ahead_bytes - work_cell * (double)nc;
             const double slot1 = 2.0 * (double)nd * (double)fsz + (out_dev ? 0.0 : (double)n_out_layers * (double)n_out * 8.0);
             const double tile_left = left / ((double)kSlots * std::max(slot1, 1.0));
-            ahead = !in_dev && !opts.skip_spinup && ctx->spin_ahead && nd > 0 && left > 0 &&
+            ahead = !in_dev && !opts.skip_spinup && nd > 0 && left > 0 &&
                     tile_left >= (double)std::min<int64_t>(nc, std::max<int64_t>(32768, nc / 16));
         }
         if (ahead) budget -= ahead_bytes;
@@ -3208,13 +3064,9 @@ struct GridJob {
         rp.w.passes = wi;
         rp.w.snap_pass = wi + pitch;
         rp.w.status = wi + 2 * pitch;
-        rp.w.frost = wi + 5 * pitch;
-        rp.w.key = (unsigned char*)(wi + 7 * pitch);
         rp.w.pitch = pitch;
         rp.lists[0] = wi + 3 * pitch;
         rp.lists[1] = wi + 4 * pitch;
-        rp.order = nullptr;
-        rp.order_w = wi + 6 * pitch;
         rp.ctl = ctl(t);
         int li = 0;
         for (int k = 0; k < 9; ++k) {
@@ -3249,7 +3101,7 @@ struct GridJob {
         k_cell_setup<<<(unsigned)((nct + 127) / 128), 128, 0, R>>>(sps[(size_t)t]);
         CU(cudaGetLastError());
         k_snow_threshold<FT><<<(unsigned)((nct + 255) / 256), 256, 0, R>>>((const FT*)rp.tc, rp.tpitch, rp.n_days, (int)nct, rp.cc,
-                                                                            rp.cpitch, rp.diag, rp.dpitch, rp.w.frost);
+                                                                            rp.cpitch, rp.diag, rp.dpitch);
         CU(cudaGetLastError());
         launches += 3;
         CU(cudaEventRecord(e.kf0, R));
@@ -3372,16 +3224,6 @@ struct GridJob {
             CU(cudaGetLastError());
             ++launches;
         }
-        if (ctx->regime_sort && nd > 0) {
-            // the finished cells in regime order (exported stragglers and, after a resume, nothing are left out)
-            CU(cudaMemsetAsync(&rp.ctl->n_ready, 0, sizeof(unsigned long long) * (1 + kRegimeKeys), R));
-            k_regime_count<<<(unsigned)((nct + 255) / 256), 256, 0, R>>>(rp);
-            k_regime_scan<<<1, 1, 0, R>>>(rp.ctl);
-            k_regime_scatter<<<(unsigned)((nct + 255) / 256), 256, 0, R>>>(rp);
-            CU(cudaGetLastError());
-            launches += 3;
-            rp.order = rp.order_w;
-        }
         CU(cudaEventRecord(e.kb0, R));
         launch_bulk<FT>(rp, monthly, R);
         CU(cudaGetLastError());
@@ -3480,7 +3322,7 @@ struct GridJob {
         CU(cudaEventRecord(ev_begin, ctx->s_h2d));
         for (auto s : ctx->s_run) CU(cudaStreamWaitEvent(s, ev_begin, 0));  // (idle streams included: harmless)
         for (int64_t t = 0; t < n_tiles; ++t) setup_params(t);
-        if (in_dev && out_dev && ctx->two_pass) {
+        if (in_dev && out_dev) {
             // resident data: every tile's spin-up first, so that the stragglers (up to 1000 sequential year
             // passes) start as early as possible and run beside the daily integration of all tiles
             for (int64_t t = 0; t < n_tiles; ++t) {

@@ -39,13 +39,9 @@
 #ifndef SPLASH_LEVEL
 #define SPLASH_LEVEL 1
 #endif
-// the two halves of level 1 can be switched separately (bisecting numerical differences)
-#ifndef SPLASH_L1_POW
+// the two halves of level 1
 #define SPLASH_L1_POW (SPLASH_LEVEL >= 1)    // x^y as exp(y*log(x)) with shared logarithms
-#endif
-#ifndef SPLASH_L1_RECIP
 #define SPLASH_L1_RECIP (SPLASH_LEVEL >= 1)  // reciprocals of per-cell constants, consistent theta scaling
-#endif
 // SPLASH_FAST_STATE: the uniform kernels' state half through day_state_fast (branch-light, same bits) with day_state as
 // the fallback; the straggler chain has its own switch (SPLASH_CHAIN_FAST, splash_cuda.cu)
 #ifndef SPLASH_FAST_STATE
@@ -169,7 +165,7 @@ struct DayOut {
 // One shared copy of each transcendental instead of ~25 inlined expansions: the day step is a
 // single long loop body and its code size, not its arithmetic, was the first bottleneck (ncu:
 // 48 % of warp-stall samples were `no_instruction` with a 91 KB kernel, profiles/README.md).
-#if SPLASH_LEVEL >= 1 && !defined(SPLASH_LIBDEVICE_MATH)
+#if SPLASH_LEVEL >= 1
 using fm::f_acos;  // splash_math.cuh: coefficients in __constant__ memory instead of 64-bit immediates
 using fm::f_exp;
 using fm::f_log;
@@ -205,18 +201,16 @@ __device__ __forceinline__ double snow_age_factor(double nd) {
 // sin(180 * pir) = sin(fl(pi)) = 1.2246467991473532e-16.
 #define SPLASH_SIN_180 kD.sin_180
 
-// How the state half of the day step reaches its transcendentals.  MathShared: calls of the shared
-// out-of-line copies (the throughput kernels, where 16 warps per SM share the instruction cache).
-// MathInline: the same algorithms expanded in place -- no call, no argument shuffling -- for the
-// straggler chain (k_pool_spin), where one warp per scheduler runs a dependent chain and every
-// instruction issued is latency.  Both evaluate identical operation sequences: results are bit-equal.
+// How the day step reaches its transcendentals.  MathShared: calls of the shared out-of-line copies.
+// MathInline: the same algorithms expanded in place -- no call, no argument shuffling -- what the day-loop
+// kernels use.  Both evaluate identical operation sequences: results are bit-equal.
 struct MathShared {
     static __device__ __forceinline__ double exp(double x) { return f_exp(x); }
     static __device__ __forceinline__ double log(double x) { return f_log(x); }
     static __device__ __forceinline__ double acos(double x) { return f_acos(x); }
     static __device__ __forceinline__ double sin(double x) { return f_sin(x); }
 };
-#if SPLASH_LEVEL >= 1 && !defined(SPLASH_LIBDEVICE_MATH)
+#if SPLASH_LEVEL >= 1
 struct MathInline {
     static __device__ __forceinline__ double exp(double x) { return fm::exp_core(x); }
     static __device__ __forceinline__ double log(double x) { return fm::log_core(x); }
@@ -1393,9 +1387,7 @@ template <class M, class CC>
 __device__ __forceinline__ bool day_state_auto(const CC& cc, const DayPre& q, CellState& st, DayOut& o, bool try_fast = true) {
     bool done = false;
     if (try_fast) done = day_state_fast<M>(cc, q, st, o);
-#ifndef SPLASH_FAST_NOFALLBACK  // (defined for timing experiments only: wrong results on the days the fast route declines)
     if (!done) day_state<M>(cc, q, st, o);
-#endif
     return done;
 }
 #else
@@ -1409,27 +1401,21 @@ __device__ __forceinline__ bool day_state_auto(const CC& cc, const DayPre& q, Ce
 //   st     state in/out;  o  fluxes of the day;  rain_out / snowfall_out  the partitioned precipitation
 //   (for the aridity index and the occurrence flags)
 // The uniform kernels expand the transcendentals in place, as the chain kernel does (measured +6 % over the shared
-// out-of-line copies once the literals moved to constant memory: no argument shuffling, no call / return;
-// -DSPLASH_SHARED_MATH restores the shared copies).  Results are bit-equal either way.
-#ifdef SPLASH_SHARED_MATH
-using DayMath = MathShared;
-#else
-using DayMath = MathInline;
-#endif
+// out-of-line copies once the literals moved to constant memory: no argument shuffling, no call / return).
 
 template <class CC>
 __device__ __forceinline__ void splash_day(const CC& cc, const DayTab& dt, const MonthTab& mt, double sw_in, double tc,
                                            double pn, CellState& st, DayOut& o, double& rain_out,
                                            double& snowfall_out) {
     DayPre q;
-    day_forcing<DayMath>(cc, dt, mt, sw_in, tc, pn, q);
+    day_forcing<MathInline>(cc, dt, mt, sw_in, tc, pn, q);
     rain_out = q.rain;
     snowfall_out = q.snowfall;
 #if SPLASH_FAST_STATE
-    day_forcing_recession<DayMath>(cc, q);
-    day_state_auto<DayMath>(cc, q, st, o);
+    day_forcing_recession<MathInline>(cc, q);
+    day_state_auto<MathInline>(cc, q, st, o);
 #else
-    day_state<DayMath>(cc, q, st, o);
+    day_state<MathInline>(cc, q, st, o);
 #endif
 }
 

@@ -1,5 +1,5 @@
 """Development aid: builds named variants of libsplash_cuda.so (extra nvcc flags) into build/variants/ in parallel, for
-A/B timing on the GPU box with SPLASH_CUDA_LIB=<path> (tools/jobs/*.sh).  usage: build_variants.py name=flags ..."""
+A/B timing on the GPU with SPLASH_CUDA_LIB=<path> (tools/knob_bench.py).  usage: build_variants.py name=flags ..."""
 import os
 import subprocess
 import sys

@@ -1,8 +1,7 @@
 """Development aid: the resident benchmark workload under different runtime knobs of the library
-(SPLASH_RUN_STREAMS, SPLASH_POOL_STAGE1, SPLASH_TWO_PASS, SPLASH_ROUNDS_RT, SPLASH_REGIME_SORT ... are read at
-context creation) and, with LIB=path, under different builds of it.
-usage: knob_bench.py <cells> <years> "K1=V1,K2=V2" "K1=V3" ...   (one timed call per setting, after one warm-up;
-       a setting may carry LIB=<path to a variant libsplash_cuda.so>: run it in a fresh process via tools/knob_sweep.sh)"""
+(SPLASH_POOL_STAGE1, SPLASH_ROUNDS_RT, SPLASH_CHAIN_FAST ... are read at context creation) and, with
+SPLASH_CUDA_LIB=<path to a variant libsplash_cuda.so> in the environment of the process, under another build of it.
+usage: knob_bench.py <cells> <years> "K1=V1,K2=V2" "K1=V3" ...   (one timed call per setting, after one warm-up)"""
 import json
 import os
 import sys
